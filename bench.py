@@ -2,7 +2,7 @@
 """bench.py - FP8 attention forward throughput on B200 (the metric of BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload C2_flux|C3_llama|C1|C4_video]
+                    [--workload C2_flux|C3_llama|C1|C4_video] [--dump-outputs DIR]
 
 One "step" = one call of the public entry point ``quantum_attn.fp8_attn_func(q, k, v)`` on 16-bit inputs that are
 already resident in HBM: dynamic FP8 quantisation of Q/K/V plus the fused attention kernel - the same thing the
@@ -117,8 +117,9 @@ class ClockSampler(threading.Thread):
         }
 
 
-def cpu_reference_leg(workload, budget_s=12.0):
-    """Time the reference's op definition on the host cores over a bounded sample of heads of the workload."""
+def cpu_reference_leg(workload, budget_s=12.0, steps=None, warmup=1):
+    """Time the reference's op definition on the host cores over a bounded sample of heads of the workload: ``steps``
+    timed runs after ``warmup`` untimed ones, or, without ``steps``, as many runs (3 to 50) as fit in ``budget_s``."""
     import oracle
 
     B, H, S, D, causal = WORKLOADS[workload]
@@ -132,10 +133,12 @@ def cpu_reference_leg(workload, budget_s=12.0):
     q8 = torch.from_numpy(q8b).view(torch.float8_e4m3fn)
     k8 = torch.from_numpy(k8b).view(torch.float8_e4m3fn)
     sq, sk, vf = torch.from_numpy(sq), torch.from_numpy(sk), v.float()
-    oracle.cpu_reference_step(q8, k8, vf, sq, sk, is_causal=causal)  # warm-up
+    for _ in range(warmup):
+        oracle.cpu_reference_step(q8, k8, vf, sq, sk, is_causal=causal)
     times = []
     t_start = time.perf_counter()
-    while len(times) < 3 or (time.perf_counter() - t_start < budget_s and len(times) < 50):
+    while (len(times) < steps if steps is not None else
+           len(times) < 3 or (time.perf_counter() - t_start < budget_s and len(times) < 50)):
         t0 = time.perf_counter()
         oracle.cpu_reference_step(q8, k8, vf, sq, sk, is_causal=causal)
         times.append(time.perf_counter() - t0)
@@ -179,6 +182,23 @@ def _claim_stdout():
     real = os.fdopen(os.dup(1), "w")
     os.dup2(2, 1)
     return real
+
+
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(dirname, out):
+    """Write ``out`` to dirname/out.npy as float32: whole when it fits in DUMP_BYTES, else the rows of its [B*H*S, D]
+    view picked by torch.randperm under seed 0, in ascending order (the same rows for the same shape in every run)."""
+    import numpy as np
+
+    rows = out.reshape(-1, out.shape[-1])
+    keep = (DUMP_BYTES - 4096) // (4 * rows.shape[1])  # (4096: room for the .npy header)
+    if rows.shape[0] > keep:
+        idx = torch.randperm(rows.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        out = rows[idx.to(rows.device)]
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "out.npy"), out.float().cpu().numpy())
 
 
 def accuracy_vs_sdpa(q, k, v, causal, out, heads=(0, -1), v_16bit=False):
@@ -532,8 +552,13 @@ def main():
     out = _claim_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=None)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps (default 1000, or 30 for sequences over 16k tokens); the reference arm times this "
+                         "many runs of its sample")
     ap.add_argument("--warmup", type=int, default=20)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (rank 0) to DIR/out.npy as float32; "
+                         "an output over 64 MB is cut to its rows [B*H*S, D] of a seed-0 sample, in order")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="C2_flux", choices=sorted(WORKLOADS))
     ap.add_argument("--event-every", type=int, default=None,
@@ -556,6 +581,10 @@ def main():
     ring = args.workload == "C4_video" and world > 1
     if args.steps is None:
         args.steps = 1000 if S <= 16384 else 30
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.event_every is None:
         args.event_every = 8 if args.steps >= 100 else 4
     if S > 16384:
@@ -593,7 +622,7 @@ def main():
         if rank != 0:
             return
         W = max(args.warmup, 0)
-        leg = cpu_reference_leg(args.workload, budget_s=min(60.0, 3.0 * max(1, args.steps)))
+        leg = cpu_reference_leg(args.workload, steps=args.steps, warmup=W)
         line = {
             "impl": "reference", "metric": METRIC, "value": leg["value"], "unit": UNIT, "n_gpus": args.gpus,
             "steps": args.steps, "warmup": W, "ms_per_step": leg["seconds_per_sample"] * 1e3,
@@ -671,7 +700,9 @@ def main():
     for i in range(args.steps):
         # the attention launch of every `--event-every`-th step is bracketed by CUDA events (roofline.achieved)
         _native.attn_events = ev_list if i % args.event_every == 0 else None
-        step(i)
+        last_out = step(i)
+        if i + 1 < args.steps:
+            del last_out  # (freed as it returns, so the allocator serves every step from the same cached blocks)
     _native.attn_events = ev_list
     e1.record()
     launches = _native.launch_total - launches0
@@ -693,6 +724,9 @@ def main():
                               f"the timed region and {extra_steps} identical untimed steps right after it")
     events, _native.attn_events = _native.attn_events, None
     attn_ms = statistics.mean(a.elapsed_time(b) for a, b in events)
+    if rank == 0 and args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, last_out)
+    del last_out
 
     if dist is not None:
         t = torch.tensor([total_ms], device=dev, dtype=torch.float64)

@@ -1,7 +1,7 @@
 """Generate tests/golden/*.npz by running the REFERENCE's own pure-torch pieces on CPU in the build container.
 
-Run once, here (needs /root/reference; never at test time on the GPU box):
-    python oracle/gen_golden.py
+Run once, with a checkout of the reference (never at test time):
+    python oracle/gen_golden.py <reference checkout>/src
 
 What is recorded
   * quantize_{head,token}.npz - inputs (bf16 bit patterns) and the outputs of the reference's
@@ -20,16 +20,15 @@ import sys
 import numpy as np
 import torch
 
-REF = "/root/reference/src"
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tests", "golden")
 
 
-def import_reference():
+def import_reference(ref_src):
     import torch._inductor.utils as iu
 
     if not hasattr(iu, "use_max_autotune"):
         iu.use_max_autotune = lambda: False
-    sys.path.insert(0, REF)
+    sys.path.insert(0, ref_src)
     import quantum_attn  # noqa: F401
     from quantum_attn import nn as ref_nn, ops as ref_ops
 
@@ -40,8 +39,8 @@ def bf16_bits(t):
     return t.contiguous().view(torch.int16).numpy().copy()
 
 
-def main():
-    ref_nn, ref_ops = import_reference()
+def main(ref_src):
+    ref_nn, ref_ops = import_reference(ref_src)
     os.makedirs(OUT, exist_ok=True)
     g = torch.Generator(device="cpu").manual_seed(1234)
 
@@ -104,6 +103,9 @@ def main():
         v = torch.randn(B, Hkv, Skv, D, generator=g16).to(dtype)
         out_16 = ref_ops._attention_forward(q, k, v, is_causal=causal)
         out_fp32 = ref_ops._attention_forward(q.float(), k.float(), v.float(), is_causal=causal)
+        # heads are independent: the B = 2 fixture keeps head 0 of each batch element, so that its file stays under 1 MB
+        h = 1 if name == "attn16_d128_fp16_causal" else Hq
+        q, k, v, out_16, out_fp32 = (t[:, :h] for t in (q, k, v, out_16, out_fp32))
         np.savez_compressed(
             os.path.join(OUT, f"{name}.npz"),
             q_bits=bf16_bits(q), k_bits=bf16_bits(k), v_bits=bf16_bits(v),  # int16 views (bf16 or fp16 bit patterns)
@@ -116,4 +118,6 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        raise SystemExit("usage: python oracle/gen_golden.py <reference checkout>/src")
+    main(sys.argv[1])

@@ -63,5 +63,36 @@ def test_reference_arm_runs_on_the_host_cores_with_the_same_config():
     _check_common(d)
     assert d["impl"] == "reference" and d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
     assert d["cpu_baseline"]["value"] == d["value"] == d["e2e"]["value"]
+    assert d["steps"] == 1 and "median of 1 runs" in d["cpu_baseline"]["sample"]  # --steps is the number of timed runs
     ours = json.load(open(os.path.join(ROOT, "profiles", "r02_bench_c2_driver.json")))
     assert set(d["config"]) == set(ours["config"]) and d["config"]["workload"] == ours["config"]["workload"]
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--impl", "reference", "--dump-outputs"]])
+def test_bench_rejects_what_it_cannot_honour(argv, tmp_path):
+    if argv[-1] == "--dump-outputs":
+        argv = argv + [str(tmp_path / "dump")]
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *argv], capture_output=True, text=True,
+                         timeout=600, cwd=ROOT)
+    assert out.returncode == 2 and out.stdout == "", out.stderr[-2000:]
+    assert not os.path.exists(tmp_path / "dump")
+
+
+def test_dump_outputs_writes_float32_whole_or_a_fixed_sample_of_rows(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+
+    import bench
+
+    out = torch.randn(2, 3, 50, 64, generator=torch.Generator().manual_seed(0)).to(torch.bfloat16)
+    bench.dump_outputs(str(tmp_path / "whole"), out)
+    whole = np.load(tmp_path / "whole" / "out.npy")
+    assert whole.dtype == np.float32 and np.array_equal(whole, out.float().numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4096 + 4 * 64 * 10)  # room for 10 rows of D = 64
+    for name in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / name), out)
+    a, b = np.load(tmp_path / "a" / "out.npy"), np.load(tmp_path / "b" / "out.npy")
+    assert a.dtype == np.float32 and a.shape == (10, 64) and np.array_equal(a, b)
+    rows = whole.reshape(-1, 64)
+    idx = [int(np.flatnonzero((rows == r).all(1))[0]) for r in a]
+    assert idx == sorted(set(idx))  # distinct rows of the output, in their order
