@@ -118,7 +118,11 @@ int qa_quantize_fp8(int n_tensors, const void* const* x, int x_dtype, const int6
  *               results across sequence shards); NULL to skip.  The reference leaves this output commented out
  *               (src/quantum_attn/tk/attention.py:333-346).  In QA_P_E4M3 mode the sum is taken over the probabilities
  *               as rounded to e4m3 - the weights that multiply V and normalise `out` - so it can differ from the
- *               exact log-sum-exp by up to about 1e-2; merging partial results with it reproduces the one-launch result.
+ *               exact log-sum-exp by up to ln(1 + 2^-4) ~= 0.061, plus ~2e-3 from the exponentials.  That bound holds
+ *               while the keys whose weight falls under e4m3's normal range (more than 10 log2 units below the row
+ *               maximum) carry a negligible share of the row sum; it is reached by a row dominated by one key whose
+ *               weight sits up to TAU = 4 log2 units above the stale running maximum.  Merging partial results with
+ *               it reproduces the one-launch result.
  *   sm_scale    softmax scale; pass 1/sqrt(D) for the reference's behaviour (src/quantum_attn/tk/attention.py:208-210)
  *   Hq % Hkv == 0 (GQA: kv head = q head / (Hq/Hkv)); D in {64, 128, 256}; causal mask is top-left aligned.
  */

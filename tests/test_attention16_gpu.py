@@ -53,6 +53,15 @@ def test_golden_fixtures_from_reference(golden_dir, name):
     (1, 2, 2100, 2100, 256),   # D = 256 runs a one-stage K/V ring: many tiles through the same slot
     (1, 1, 1, 1, 128),         # degenerate
     (1, 1, 129, 3, 64),
+    # where the per-tile step counts, the first masked step and the all-padding second query tile change
+    (1, 2, 64, 64, 128),
+    (1, 2, 65, 65, 256),
+    (1, 2, 128, 128, 64),
+    (1, 2, 129, 129, 128),
+    (1, 2, 256, 256, 256),
+    (1, 2, 257, 257, 64),
+    (1, 2, 257, 65, 256),
+    (1, 2, 1, 4097, 128),
 ])
 def test_parity_sweep(B, H, Sq, Skv, D, causal):
     if causal and Sq != Skv:

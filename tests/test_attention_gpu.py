@@ -119,6 +119,15 @@ def test_golden_token_wise(golden_dir):
     (1, 2, 1000, 1000, 256),
     (1, 1, 1, 1, 128),         # degenerate
     (1, 1, 129, 3, 64),
+    # where the per-tile step counts, the first masked step and the all-padding second query tile change
+    (1, 2, 64, 64, 64),
+    (1, 2, 65, 65, 128),
+    (1, 2, 128, 128, 256),
+    (1, 2, 129, 129, 64),
+    (1, 2, 256, 256, 128),
+    (1, 2, 257, 257, 256),
+    (1, 2, 257, 65, 128),
+    (1, 2, 1, 4097, 64),
 ])
 def test_parity_sweep(B, H, Sq, Skv, D, causal, pv):
     if causal and Sq != Skv:
