@@ -345,3 +345,19 @@ CASES = [
     Case("spike_d64_causal", lambda t: spike(1, 3 + 5 / 64), 64, 1000, 1000, True, ()),
 ]
 LONG = Case("c4_tail", c4_tail, 128, 256, 75600, False, tuple(range(1171, 1177)) + (1181,))
+
+# Causal problems with Sq != Skv (top-left mask: row i sees keys 0 .. min(i, Skv - 1)), run by
+# tests/test_causal_rectangular_gpu.py.  RECT_WARPS: the 32-row warps that must rescale, where the design pins them.
+RECT_CASES = [
+    # level-60 keys from key 640 on, past every row's diagonal (rows < 512): no rescale, and a kernel that reads them
+    # (a step too far, or a bottom-right mask) is off by orders of magnitude
+    Case("rect_j10_60_512x2048_d128", lambda t: jump(10, 60.0), 128, 512, 2048, True, ()),
+    # keys 256-319 (step 4) only reach rows >= 256: tiles 0 and 1 stop at 2 and 4 steps, warps 8-31 rescale
+    Case("rect_j4_3tau_1024x320_d128", lambda t: jump(4, 3 * t), 128, 1024, 320, True, (4,)),
+    Case("rect_j4_3tau_1024x320_d256", lambda t: jump(4, 3 * t), 256, 1024, 320, True, (4,)),
+    # the ragged last step (keys 256-299 of 300): a spike that rows >= 261 see, and a jump that rows >= 256 see
+    Case("rect_spike_ragged_1000x300_d64", lambda t: spike(4, 3 + 5 / 64), 64, 1000, 300, True, ()),
+    Case("rect_jlast_ragged_1000x300_d256", lambda t: jump(4, t + 0.25), 256, 1000, 300, True, (4,)),
+]
+RECT_WARPS = {"rect_j4_3tau_1024x320_d128": range(8, 32), "rect_j4_3tau_1024x320_d256": range(8, 32),
+              "rect_jlast_ragged_1000x300_d256": range(8, 32)}

@@ -47,7 +47,7 @@ def test_golden_fixtures_from_reference(golden_dir, name):
     (1, 2, 1024, 1024, 128),
     (1, 2, 999, 999, 128),     # ragged (the reference's 16-bit sweep uses 999, tests/test_interface.py:64-65)
     (1, 2, 999, 999, 64),
-    (1, 2, 999, 1024, 128),    # Sq != Skv (non-causal only, as in the reference)
+    (1, 2, 999, 1024, 128),    # Sq != Skv (causal: the top-left mask, as torch SDPA's is_causal)
     (1, 2, 1024, 999, 256),
     (1, 2, 999, 999, 256),
     (1, 2, 2100, 2100, 256),   # D = 256 runs a one-stage K/V ring: many tiles through the same slot
@@ -64,8 +64,6 @@ def test_golden_fixtures_from_reference(golden_dir, name):
     (1, 2, 1, 4097, 128),
 ])
 def test_parity_sweep(B, H, Sq, Skv, D, causal):
-    if causal and Sq != Skv:
-        pytest.skip("Causal attention is only supported for S_Q == S_KV")
     q, k, v = oracle.make_qkv(B, H, Sq, Skv, D, seed=Sq + D)
     out = _native.attn_fwd(q.cuda(), k.cuda(), v.cuda(), is_causal=causal, sm_scale=1.0 / math.sqrt(D))
     check(out, oracle.sdpa_ref(q, k, v, is_causal=causal), f"{(B, H, Sq, Skv, D, causal)}")

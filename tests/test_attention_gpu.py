@@ -114,7 +114,7 @@ def test_golden_token_wise(golden_dir):
     (1, 2, 1024, 1024, 128),
     (1, 2, 1000, 1000, 128),   # ragged
     (1, 2, 999, 999, 64),
-    (1, 2, 1000, 1024, 128),   # Sq != Skv (non-causal only, as in the reference)
+    (1, 2, 1000, 1024, 128),   # Sq != Skv (causal: the top-left mask, as torch SDPA's is_causal)
     (1, 2, 1024, 1000, 256),
     (1, 2, 1000, 1000, 256),
     (1, 1, 1, 1, 128),         # degenerate
@@ -130,8 +130,6 @@ def test_golden_token_wise(golden_dir):
     (1, 2, 1, 4097, 64),
 ])
 def test_parity_sweep(B, H, Sq, Skv, D, causal, pv):
-    if causal and Sq != Skv:
-        pytest.skip("Causal attention is only supported for S_Q == S_KV")
     q, k, v = oracle.make_qkv(B, H, Sq, Skv, D, seed=Sq + D)
     out, ref, _ = run_native(q, k, v, causal=causal, pv=pv)
     check(out, ref, pv, f"{(B, H, Sq, Skv, D, causal, pv)}")

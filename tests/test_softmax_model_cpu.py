@@ -37,7 +37,7 @@ def _check_bytes(L, token):
 
 
 @pytest.mark.parametrize("fam", ["16bit", "e4m3"])
-@pytest.mark.parametrize("case", sm.CASES, ids=[c.name for c in sm.CASES])
+@pytest.mark.parametrize("case", sm.CASES + sm.RECT_CASES, ids=[c.name for c in sm.CASES + sm.RECT_CASES])
 def test_landscape_drives_the_intended_rescales(case, fam):
     tau, koff = sm.tau_koff(fam == "16bit")
     design = case.make(tau)
@@ -55,6 +55,20 @@ def test_landscape_drives_the_intended_rescales(case, fam):
         assert 2.0**r.max_exp <= sm.E4M3_P_HEADROOM <= sm.E4M3_P_MAX
     if "below" in case.name:  # the headroom cases come within 1/4 + 2 ETA of it
         assert r.max_exp >= koff + tau - 0.25 - 2 * sm.ETA
+
+
+@pytest.mark.parametrize("fam", ["16bit", "e4m3"])
+@pytest.mark.parametrize("case", sm.RECT_CASES, ids=[c.name for c in sm.RECT_CASES])
+def test_rectangular_landscape_rescales_the_intended_warps(case, fam):
+    """Causal with Sq != Skv: only the warps whose rows reach the raised keys rescale, and keys past every row's
+    diagonal leave the masked LSE alone while they would dominate it unmasked."""
+    tau, _ = sm.tau_koff(fam == "16bit")
+    L = sm.landscape(case.make(tau), Sq=case.Sq, Skv=case.Skv, D=case.D, seed=1)
+    r = sm.rescale_events(L.x, v16=fam == "16bit", causal=True, D=case.D)
+    assert {w for (_, _, w, _) in r.events} == set(sm.RECT_WARPS.get(case.name, ())), case.name
+    if case.Sq < case.Skv:
+        assert sm.logsumexp_ref(L.x, causal=True).max() < math.log(case.Sq) + sm.ETA  # Sq keys of level ~0 at most
+        assert sm.logsumexp_ref(L.x, causal=False).min() > 59 * sm.LN2
 
 
 def test_long_landscape_drives_the_intended_rescales():
