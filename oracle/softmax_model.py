@@ -42,13 +42,13 @@ CH_NOISE = 6
 
 
 def tau_koff(v16: bool):
-    """(TAU, KOFF) of the kernel: mirrors AttnCfg::TAU / AttnCfg::KOFF (attn_fwd_kernel.cuh:230-232).  p' =
+    """(TAU, KOFF) of the kernel: mirrors AttnCfg::TAU / AttnCfg::KOFF (attn_fwd_kernel.cuh:131-133).  p' =
     2^KOFF * exp2(s - m_used), and m_used may lag the true row maximum by up to TAU (log2 units) before a rescale."""
     return (8.0, 0.0) if v16 else (4.0, 4.0)
 
 
 def n_tiles_per_cta(D: int) -> int:
-    """Query tiles per CTA (AttnCfg::NQ in the default build): two for D <= 128, one at D = 256."""
+    """Query tiles per CTA (AttnCfg::NQ): two for D <= 128, one at D = 256."""
     return 2 if D <= 128 else 1
 
 

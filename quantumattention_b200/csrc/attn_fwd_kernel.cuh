@@ -51,81 +51,14 @@ constexpr int BM = 128;  // query rows per tile (= TMEM lanes)
 constexpr int BN = 128;  // keys per K/V shared-memory tile (one TMA box)
 constexpr int BS = 64;   // keys per softmax / MMA step (half a tile)
 constexpr float kLog2e = 1.4426950408889634f;
+constexpr int kTmemCols = 512;  // one CTA per SM owns all of tensor memory
+// setmaxnreg moves registers inside the allocation the CTA was launched with (two query tiles: 12 warps x 168 =
+// 8 softmax warps x 224 + 4 MMA / TMA warps x 56)
+constexpr int kRegSoftmax = 224, kRegOther = 56;
 
-#ifndef QA_POLY_NUM
-#define QA_POLY_NUM 2  // of every 8 pairs of exponentials, how many run on the FMA pipe instead of MUFU
-#endif
-#ifndef QA_LOADQ
-#define QA_LOADQ 8    // S_{j+1} is pulled into registers after this many (of 16) quads of step j's exponentials
-#endif
-#ifndef QA_MMASUM
-#define QA_MMASUM 1    // single-e4m3 P mode: row sums of P come from the tensor core (P x ones) instead of 64 FADDs per step
-#endif
-#ifndef QA_DIRECT_STORE
-#define QA_DIRECT_STORE 1  // epilogue writes O rows straight from registers (256-bit stores) instead of smem + TMA
-#endif
-#ifndef QA_PUBQ
-#define QA_PUBQ 2      // P_{j-1} (stored at the end of step j-1) is published after this many quads of step j
-#endif
-#ifndef QA_LDWAITQ
-#define QA_LDWAITQ 4   // quads of exponentials between the TMEM load of S_{j+1} and the wait for it
-#endif
-#ifndef QA_PROBEQ
-#define QA_PROBEQ 0    // > 0: the barrier of S_{j+1} is probed this many quads before the load (hides the probe's latency)
-#endif
-#ifndef QA_SOLO
-#define QA_SOLO 0      // 1: one query tile per CTA and two CTAs per SM for D <= 128 (see AttnCfg::SOLO)
-#endif
-#ifndef QA_MMASUM_D256
-#define QA_MMASUM_D256 0
-#endif
-#ifndef QA_POLY_MS_D64
-#define QA_POLY_MS_D64 3
-#endif
-#ifndef QA_POLY_MS_D256
-#define QA_POLY_MS_D256 1
-#endif
-#ifndef QA_POLY_D256
-#define QA_POLY_D256 2
-#endif
-#ifndef QA_POLY_P16
-#define QA_POLY_P16 QA_POLY_NUM  // 16-bit P mode (the default mode), D <= 128; C2 kernel 177.8 / 173.0 / 167.7 / 173.0 / 175.5 us at 0..4
-#endif
-#ifndef QA_H2POLY
-#define QA_H2POLY 0    // 1: polynomial exponentials in packed half precision (measured slower: the extra ALU-pipe work)
-#endif
-#ifndef QA_H2POLY_NUM
-#define QA_H2POLY_NUM 5  // of every 8 pairs of exponentials, how many take the half-precision polynomial (single-e4m3 mode)
-#endif
-#ifndef QA_DECIDEQ
-#define QA_DECIDEQ 1   // quads of exponentials left when the rescale decision for the next step is taken
-#endif
-#ifndef QA_QTMEM
-#define QA_QTMEM 1     // e4m3 Q in tensor memory, Q K^T as a TS-form MMA: 1 = where it pays (D = 256), 2 = everywhere, 0 = nowhere
-#endif
 #ifndef QA_SYNCCHECK
 #define QA_SYNCCHECK 0  // 1: the softmax threads wait for EVERY PV_{j-1} (compute-sanitizer synccheck flags barrier phases nobody
                         // observed; the shipping kernel only waits for a PV where its completion matters - rescale, last step)
-#endif
-#ifndef QA_FORCE_PBUFS1
-#define QA_FORCE_PBUFS1 0  // experiment: one P buffer without Q in TMEM (measured: C2 172.4 -> 180.6 us)
-#endif
-// Developer ablations (WRONG results, timing only; scripts/gpu_r02_abl.sh): issue only a part of the MMAs / evaluate only a
-// part of the exponentials, to measure how the step time responds to each resource (DESIGN.md section 4.2).
-#ifndef QA_ABL_QK
-#define QA_ABL_QK 0    // > 0: Q K^T issues only this many of its K slices
-#endif
-#ifndef QA_ABL_PV
-#define QA_ABL_PV 0    // > 0: P V issues only this many of its MMAs per step
-#endif
-#ifndef QA_ABL_EXP
-#define QA_ABL_EXP 0   // > 0: only the first this-many pairs (of 32) of a step's scores go through scale + exp2
-#endif
-#ifndef QA_WARP_ARRIVE
-#define QA_WARP_ARRIVE 0  // 1: one elected lane per softmax warp arrives on s_free / p_full / q_full (4 arrivals instead of 128)
-#endif
-#ifndef QA_SPLIT
-#define QA_SPLIT 0     // 1: TWO softmax threads per query row (each owns half of a step's 64 columns): 4 softmax warps per scheduler
 #endif
 
 // QK16_: Q and K stay 16-bit (bf16 / fp16) and QK^T runs as kind::f16 - the reference's `attn_func` path
@@ -141,12 +74,8 @@ struct AttnCfg {
     static constexpr bool PF16 = PF16_;
     static constexpr bool V16 = (PMODE_ == QA_P_16BIT);
     static_assert(!QK16_ || V16, "16-bit Q/K go with 16-bit P and V");
-    // Two shapes of CTA.  PAIR: two query tiles share the K / V tiles of one CTA (one CTA per SM, all 512 TMEM columns).
-    // SOLO (-DQA_SOLO=1, D <= 128, 8-bit Q/K/V): one query tile per CTA, 256 TMEM columns, two CTAs per SM - each tile
-    // loads its own K / V, but one CTA's prologue / epilogue overlaps the other's main loop and causal work is dealt out
-    // in 128-row units.
-    static constexpr bool SOLO = (QA_SOLO != 0) && D_ <= 128 && !QK16_ && !(PMODE_ == QA_P_16BIT);
-    static constexpr int NQ = (D_ <= 128 && !SOLO) ? 2 : 1;  // O for two tiles does not fit TMEM at D = 256
+    // query tiles per CTA: two share the K / V tiles of one CTA, but O for two tiles does not fit TMEM at D = 256
+    static constexpr int NQ = D_ <= 128 ? 2 : 1;
     // Q in TENSOR MEMORY (D = 256).  An SS-form tcgen05.mma (A and B from shared memory) first loads its A operand - 128
     // rows x 32 bytes - which costs ~43 cycles per MMA on top of the N / 2 cycles of the product itself: measured on
     // B200 (scripts/ubench/mma_rate.cu) M128 x N64 x K32 takes 75 cycles from shared memory and 42 with A in TMEM.  Q
@@ -156,21 +85,9 @@ struct AttnCfg {
     // (16-bit P) / 510 -> 477 us (e4m3 P) on B16 S8192, causal 316 -> 289 us.  At D <= 128 the two tiles of a CTA
     // leave no columns for Q unless P goes down to one buffer, and there the tensor pipe is not what bounds the step:
     // measured SLOWER with Q in TMEM (C2 168.6 -> 184.8 us; one P buffer alone 172.4 -> 180.6 us), so those shapes
-    // keep Q in shared memory (-DQA_QTMEM=2 forces the TMEM form everywhere, =0 nowhere).  Not for 16-bit Q.
-    static constexpr bool QTMEM = (QA_QTMEM == 2 || (QA_QTMEM == 1 && D_ == 256)) && (QA_DIRECT_STORE != 0) && !QK16_ && !SOLO;
-    static constexpr int PBUFS = ((QTMEM && D_ != 256) || QA_FORCE_PBUFS1) ? 1 : 2;  // (D = 256: one tile, both P buffers fit beside Q)
-    // NH softmax threads share a query row: thread `hf` of a row owns columns [hf * CW, (hf + 1) * CW) of every 64-key
-    // step (TMEM lets the warps w and w + 4 of a tile read the same 32 lanes).  NH = 2 doubles the softmax warps per
-    // scheduler (4 instead of 2 at D <= 128), i.e. the thread-level parallelism that hides the MUFU dispatch and the
-    // dependent-issue latencies the exponential stream is bound by; the two threads of a row agree on the running
-    // maximum through a named-barrier vote per step and a shared-memory exchange on the (rare) rescales.
-    static constexpr int NH = (QA_SPLIT != 0 && !SOLO) ? 2 : 1;
-    static constexpr int CW = BS / NH;  // score columns per softmax thread and step
-    static constexpr int CTAS_PER_SM = SOLO ? 2 : 1;
-    static constexpr int TMEM_COLS = SOLO ? 256 : 512;
-    static constexpr bool REBALANCE = (NQ == 2) || SOLO;  // setmaxnreg: registers move to the softmax warps
-    // (setmaxnreg moves registers inside the allocation the CTA was launched with: 20 warps x 96 = 16 x 104 + 4 x 64)
-    static constexpr int REG_SOFTMAX = SOLO ? 216 : (NH == 2 ? 112 : 224), REG_OTHER = SOLO ? 40 : (NH == 2 ? 32 : 56);
+    // keep Q in shared memory.  Not for 16-bit Q.
+    static constexpr bool QTMEM = D_ == 256 && !QK16_;
+    static constexpr bool REBALANCE = NQ == 2;  // setmaxnreg: registers move to the softmax warps
     static constexpr int VB = V16 ? 2 : 1;          // bytes per V element
     static constexpr int QB = QK16_ ? 2 : 1;        // bytes per Q / K element
     // shared-memory tiles are stored as "boxes" whose rows are one swizzle span (<= 128 bytes) wide
@@ -183,65 +100,44 @@ struct AttnCfg {
     static constexpr int Q_TILE = QTMEM ? 0 : BM * D_ * QB;
     static constexpr int K_TILE = BN * D_ * QB;
     static constexpr int V_TILE = BN * D_ * VB;
-    static constexpr int O_BOXES = D_ / 64;  // 16-bit output, 64 elements = 128 bytes per box row
-    static constexpr int O_TILE = BM * D_ * 2;
-    static constexpr bool DIRECT_STORE = (QA_DIRECT_STORE != 0);
-    static constexpr int STAGES = SOLO ? (D_ == 64 ? 4 : 2)
-                                  : QK16_ ? (D_ == 64 ? 4 : (D_ == 128 ? 2 : 1))
-                                          : ((D_ == 64) ? 4 : (D_ == 128 ? ((V16 && !DIRECT_STORE) ? 2 : (QTMEM ? 4 : 3)) : 2));
+    static constexpr int STAGES = QK16_ ? (D_ == 64 ? 4 : (D_ == 128 ? 2 : 1)) : (D_ == 64 ? 4 : (D_ == 128 ? 3 : 2));
     static constexpr int SMEM_Q = 0;
     static constexpr int SMEM_K = SMEM_Q + NQ * Q_TILE;
     static constexpr int SMEM_V = SMEM_K + STAGES * K_TILE;
-    // O staging for the TMA-store epilogue (QA_DIRECT_STORE=0 only; the default epilogue stores rows from registers):
-    // its own region when two query tiles finish at different times; with a single tile (D = 256) every MMA has retired
-    // before the epilogue, so the dead K ring is reused; with 16-bit Q a query tile is as large as its output tile and
-    // dead once the tile's last MMA has retired, so O is staged over Q
-    static constexpr bool O_OWN = !DIRECT_STORE && NQ == 2 && !QK16_;
-    static constexpr int SMEM_O = QK16_ ? SMEM_Q : (O_OWN ? SMEM_V + STAGES * V_TILE : SMEM_K);
-    static_assert(DIRECT_STORE || QK16_ || NQ == 2 || STAGES * K_TILE >= O_TILE, "K ring too small to stage O");
-    static_assert(!QK16_ || Q_TILE == O_TILE, "O is staged over Q");
     // single-e4m3 P mode: the row sums of P are accumulated by the tensor core, L (+)= P . 1, with a constant tile of
     // e4m3 ones (0x38) as the B operand - every byte the MMA can touch holds the same value, so the tile's layout is
     // immaterial - and a 16-column accumulator per query tile in the TMEM columns the 16-bit P buffers leave unused.
-    static constexpr bool MMASUM = (QA_MMASUM != 0) && (PMODE_ == QA_P_E4M3) && !QK16_ && (D_ != 256 || QA_MMASUM_D256 != 0);
+    // Not at D = 256, where the extra MMA costs more than the FADDs it saves (DESIGN.md section 4.2).
+    static constexpr bool MMASUM = PMODE_ == QA_P_E4M3 && !QK16_ && D_ != 256;
     static constexpr int ONES_BYTES = MMASUM ? 4096 : 0;  // 32 keys x one swizzle span
-    static constexpr int SMEM_ONES = O_OWN ? SMEM_O + NQ * O_TILE : SMEM_V + STAGES * V_TILE;
-    static constexpr int SMEM_BAR = SMEM_ONES + ONES_BYTES;
-    static constexpr int SMEM_XCHG = SMEM_BAR + 512;          // split softmax: one float per (tile, share, row)
-    static constexpr int XCHG_BYTES = (NH == 2) ? NQ * 2 * 128 * 4 : 0;
+    static constexpr int SMEM_ONES = SMEM_V + STAGES * V_TILE;
+    static constexpr int SMEM_BAR = SMEM_ONES + ONES_BYTES;  // struct Barriers, 512 bytes reserved
     // per-token K scales (token-wise kernels): the 128 scales of a K / V tile ride the V ring - one 512-byte bulk copy
     // per tile next to the V boxes, completing on the same barrier - and the softmax threads read them from shared memory
-    static constexpr int SMEM_SK = SMEM_XCHG + XCHG_BYTES;
+    static constexpr int SMEM_SK = SMEM_BAR + 512;
     static constexpr int SK_BYTES = STAGES * BN * 4;
-    static constexpr int SMEM_TOTAL = SMEM_SK + SK_BYTES + 1024;  // + barriers + alignment slack
-    static_assert(SMEM_TOTAL * CTAS_PER_SM + 1024 * CTAS_PER_SM <= 233472, "shared memory budget exceeded");
-    static constexpr int NSOFT = NQ * 4 * NH;           // softmax warps
+    static constexpr int SMEM_TOTAL = SMEM_SK + SK_BYTES + 1024;  // + alignment slack
+    static_assert(SMEM_TOTAL + 1024 <= 233472, "shared memory budget exceeded");
+    static constexpr int NSOFT = NQ * 4;                // softmax warps
     static constexpr int NTHREADS = (NSOFT + 4) * 32;   // softmax warpgroups + one warpgroup holding the MMA / TMA warps
-    static_assert(NH == 1 || DIRECT_STORE, "the split softmax writes its output rows from registers");
     // TMEM columns
     static constexpr int TM_S = 0;                        // S_t at t * 128 (64 columns)
     static constexpr int TM_P = 64;                       // P(t, b) at t * 128 + 64 + b * 32
-    static constexpr int TM_O = SOLO ? 128 : 256;         // O_t at 256 + t * 128 (D <= 128), single O at D = 256; SOLO: 128
+    static constexpr int TM_O = 256;                      // O_t at 256 + t * 128 (D <= 128), single O at D = 256
     static constexpr int TM_P_LO = 16;                    // hi/lo mode: second P tile 16 columns after the first
     static constexpr int TM_L = 80;                       // MMASUM: L_t at t * 128 + 80 (16 columns, column 0 is read)
-    // QTMEM: Q_t (D / 4 columns) behind the single P buffer: t * 128 + 96 (D <= 128), 128 at D = 256 (one tile: room)
-    static constexpr int TM_Q = (D_ == 256) ? 128 : 96;
+    static constexpr int TM_Q = 128;                      // QTMEM (D = 256, one tile): Q in the D / 4 columns after P
 
     // softmax range management: p' = 2^KOFF * exp2(s - m_used), m_used may lag the true max by <= TAU (log2 units)
     static constexpr float KOFF = V16 ? 0.f : 4.f;
     static constexpr float TAU = V16 ? 8.f : 4.f;
-    // exponentials on the FMA pipe: polynomial degree (a single e4m3 P tolerates the quadratic's 1.7e-3)
-    // Single-e4m3 mode with tensor-core row sums: the softmax threads need p' only as e4m3 bytes, so the polynomial
-    // exponentials can run in packed half precision (exp2_pair_h2).  Same accuracy, but measured SLOWER on C2 (148 us with
-    // the fp32 polynomial on 3/8 of the pairs; 156 / 158 / 168 / 180 us with the half-precision one on 4 / 5 / 6 / 8 of 8):
-    // conversions, clamp and exponent insertion land on the half-rate ALU pipe.  Off by default.
-    static constexpr bool H2POLY = (QA_H2POLY != 0) && MMASUM;
-    // The share of polynomial pairs is a per-head-dimension balance, measured with scripts/time_shape.py: at D = 64 the
-    // MUFU is the contended unit (little tensor work per score), at D = 256 a CTA has one softmax warp per scheduler,
-    // the MUFU is never contended and every polynomial is pure extra issue work.
-    static constexpr int POLY_NUM = H2POLY   ? QA_H2POLY_NUM
-                                    : MMASUM ? (D_ == 64 ? QA_POLY_MS_D64 : (D_ == 128 ? QA_POLY_NUM + 1 : QA_POLY_MS_D256))
-                                             : (D_ == 256 ? QA_POLY_D256 : (PMODE_ == QA_P_16BIT ? QA_POLY_P16 : QA_POLY_NUM));
+    // Exponentials on the FMA pipe: of every 8 pairs, POLY_NUM are evaluated as a polynomial instead of by MUFU.EX2.
+    // The share is a per-head-dimension balance, measured with scripts/time_shape.py: at D = 64 the MUFU is the contended
+    // unit (little tensor work per score), at D = 256 a CTA has one softmax warp per scheduler, the MUFU is never
+    // contended and every polynomial is pure extra issue work.  3 of 8 where the tensor core sums the rows (D = 64 and
+    // 128 with a single e4m3 P), 2 of 8 elsewhere (16-bit P mode, C2 kernel 177.8 / 173.0 / 167.7 / 173.0 / 175.5 us at
+    // 0..4 of 8).  Polynomial degree: a single e4m3 P tolerates the quadratic's 1.7e-3.
+    static constexpr int POLY_NUM = MMASUM ? 3 : 2;
     static constexpr int POLY_DEG = (PMODE_ == QA_P_E4M3) ? 2 : 3;
 };
 
@@ -278,18 +174,6 @@ struct Barriers {
 };
 static_assert(sizeof(Barriers) <= 512, "barrier block too large");
 
-// Arrival of a softmax warp on a barrier its query tile's MMA warp waits for.  The tcgen05.ld / .st the arrival vouches for
-// are warp-collective and each lane has fenced them, so after a warp sync one lane can arrive for all 32.
-constexpr int kTileArrivals = QA_WARP_ARRIVE ? 4 : 128;  // per tile and softmax thread share
-__device__ __forceinline__ void softmax_arrive(uint64_t* bar) {
-#if QA_WARP_ARRIVE
-    __syncwarp();
-    if ((threadIdx.x & 31) == 0) mbar_arrive(bar);
-#else
-    mbar_arrive(bar);
-#endif
-}
-
 template <class C>
 __device__ __forceinline__ uint32_t qk_koff(int k) {  // byte offset of the k-th 32-byte K slice inside a Q/K tile
     constexpr int per_box = C::QK_ROW / 32;
@@ -325,33 +209,14 @@ __device__ __forceinline__ float2 exp2_poly(float2 x) {
     return r;
 }
 
-// 2^x for a pair, entirely in packed half precision (one issue cycle per instruction for two elements, where the packed
-// fp32 forms take two): x is rounded to f16 (|x| < 16 here: an absolute error of 2^-7 at most, 0.5 % in 2^x - far below
-// the e4m3 step the result is rounded to), n = round(x) comes from the 1536-magic of f16 with 15 folded in so that the
-// low five mantissa bits of t are n + 15 = the biased f16 exponent of 2^n, f = x - n, 2^f by the quadratic, and the
-// scale 2^n is built by shifting those five bits into the exponent field.  x <= -15 gives exactly 0; x must stay
-// below 16 (the lazy-rescale rule keeps it below KOFF + TAU = 8).  Returns the f16x2 bits.
-__device__ __forceinline__ uint32_t exp2_pair_h2(float2 x) {
-    __half2 xh = __float22half2_rn(x);
-    xh = __hmax2(xh, __float2half2_rn(-15.f));
-    const __half2 magic = __float2half2_rn(1551.f);
-    const __half2 t = __hadd2(xh, magic);
-    const __half2 f = __hsub2(xh, __hsub2(t, magic));
-    __half2 q = __hfma2(f, __float2half2_rn(0.23842893540859222f), __float2half2_rn(0.7034479975700378f));
-    q = __hfma2(q, f, __float2half2_rn(1.0004431009292603f));
-    const uint32_t e = (*reinterpret_cast<const uint32_t*>(&t) & 0x001F001Fu) << 10;
-    const __half2 r = __hmul2(q, *reinterpret_cast<const __half2*>(&e));
-    return *reinterpret_cast<const uint32_t*>(&r);
-}
-
 __host__ __device__ constexpr bool pair_uses_poly(int i, int num) {  // spread `num` of every 8 pairs evenly
     return (((i & 7) + 1) * num) / 8 > ((i & 7) * num) / 8;
 }
 
 template <class C, bool CAUSAL, bool TOKEN>
-__global__ void __launch_bounds__(C::NTHREADS, C::CTAS_PER_SM)
+__global__ void __launch_bounds__(C::NTHREADS, 1)
 attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK,
-                const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmO, AttnParams p) {
+                const __grid_constant__ CUtensorMap tmV, AttnParams p) {
     constexpr int D = C::D;
     constexpr int NQ = C::NQ;
     extern __shared__ uint8_t smem_raw[];
@@ -382,7 +247,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
     // (everything up to the griddep_wait()s below touches no global data: it overlaps the tail of the previous kernel,
     // normally the quantiser that produces q8 / k8 / v8 and their scales)
     if (warp == 0) {
-        tmem_alloc(&bars->tmem_base, C::TMEM_COLS);
+        tmem_alloc(&bars->tmem_base, kTmemCols);
         tmem_relinquish();
     }
     if (warp == 1) {  // one barrier per lane
@@ -390,8 +255,8 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
             const int t = lane >> 1, x = lane & 1;
             if (x) mbar_init(&bars->o_full[t], 1);
             mbar_init(&bars->pv_done[t][x], 1);
-            mbar_init(&bars->p_full[t][x], kTileArrivals * C::NH);
-            mbar_init(x ? &bars->s_free[t] : &bars->s_full[t], x ? kTileArrivals * C::NH : 1);
+            mbar_init(&bars->p_full[t][x], BM);  // (s_free, p_full: every softmax thread of the tile arrives)
+            mbar_init(x ? &bars->s_free[t] : &bars->s_full[t], x ? BM : 1);
         }
         fence_barrier_init();
     }
@@ -442,7 +307,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
             mbar_init(&bars->v_full[lane], (TOKEN && !p.sk_bulk) ? 2 : 1);
             mbar_init(&bars->v_empty[lane], NQ);
         } else if (lane < 4 + NQ) {
-            mbar_init(&bars->q_full[lane - 4], C::QTMEM ? kTileArrivals : 1);  // QTMEM: the tile's 128 rows, each put there by its thread
+            mbar_init(&bars->q_full[lane - 4], C::QTMEM ? BM : 1);  // QTMEM: the tile's 128 rows, each put there by its thread
         }
         fence_barrier_init();
         __syncwarp();
@@ -450,7 +315,6 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
             tma_prefetch_desc(&tmQ);
             tma_prefetch_desc(&tmK);
             tma_prefetch_desc(&tmV);
-            tma_prefetch_desc(&tmO);
             griddep_wait();
             if (p.kv_ready != nullptr) {
                 // gated launch: this head's K / V may still be on their way (copy engines, another stream).  A bounded
@@ -499,14 +363,13 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
-    // PAIR: the CTA owns all 512 columns, so the allocation starts at column 0; SOLO: 0 or 256
-    if (!C::SOLO && bars->tmem_base != 0) __trap();
-    const uint32_t tmem = C::SOLO ? bars->tmem_base : 0u;
+    // the CTA owns all 512 columns, so the allocation starts at column 0: TMEM addresses are the TM_* offsets below
+    if (bars->tmem_base != 0) __trap();
 
     // register rebalancing (two-tile configs run 384 threads -> 168 registers each at launch): the softmax
     // warpgroups keep a whole score row per thread in registers, the MMA / TMA warps need almost nothing
     if (warp >= C::NSOFT) {
-        if constexpr (C::REBALANCE) reg_dealloc<C::REG_OTHER>();
+        if constexpr (C::REBALANCE) reg_dealloc<kRegOther>();
         if (warp == C::NSOFT + 1) {
             // =========================================================== TMA producer
             if (TOKEN && !p.sk_bulk) {
@@ -551,11 +414,11 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
             const uint64_t k_desc0 = make_smem_desc(smem_u32(smem + C::SMEM_K), 16, 8 * C::QK_ROW, qk_swz);
             const uint64_t v_desc0 = make_smem_desc(smem_u32(smem + C::SMEM_V), C::V_BOX_BYTES, 8 * C::V_ROW, v_swz);
             constexpr int KEYS_PER_PV = C::V16 ? 16 : 32;
-            const uint32_t s_t = tmem + C::TM_S + t * 128;
-            const uint32_t p_t0 = tmem + C::TM_P + t * 128;
-            const uint32_t q_t = tmem + C::TM_Q + t * 128;  // QTMEM: K slice k of Q_t = 8 columns at q_t + 8 k
-            const uint32_t o_t = tmem + C::TM_O + (NQ == 2 ? t * 128 : 0);
-            const uint32_t l_t = tmem + C::TM_L + t * 128;
+            const uint32_t s_t = C::TM_S + t * 128;
+            const uint32_t p_t0 = C::TM_P + t * 128;
+            const uint32_t q_t = C::TM_Q + t * 128;  // QTMEM: K slice k of Q_t = 8 columns at q_t + 8 k
+            const uint32_t o_t = C::TM_O + (NQ == 2 ? t * 128 : 0);
+            const uint32_t l_t = C::TM_L + t * 128;
             constexpr uint32_t idesc_l = make_idesc(0, 0, 0, 1, BM, 16);
             const uint64_t ones_desc = make_smem_desc(smem_u32(smem + C::SMEM_ONES), C::V_BOX_BYTES, 8 * C::V_ROW, v_swz);
 
@@ -563,7 +426,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
             auto issue_qk = [&](int stage, int half) {
                 const uint64_t bd = k_desc0 + uint64_t((stage * C::K_TILE + half * (BS * C::QK_ROW)) >> 4);
 #pragma unroll
-                for (int k = 0; k < (QA_ABL_QK > 0 ? QA_ABL_QK : D * C::QB / 32); ++k) {  // one MMA per 32-byte K slice (32 e4m3 / 16 bf16 elements)
+                for (int k = 0; k < D * C::QB / 32; ++k) {  // one MMA per 32-byte K slice (32 e4m3 / 16 bf16 elements)
                     if constexpr (C::QK16)
                         umma_f16_ss(s_t, q_desc + (qk_koff<C>(k) >> 4), bd + (qk_koff<C>(k) >> 4), idesc_qk, k > 0);
                     else if constexpr (C::QTMEM)
@@ -574,10 +437,10 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
             };
             // O_t (+)= P(t, half) . V[64 keys]
             auto issue_pv = [&](int stage, int half, bool acc) {
-                const uint32_t p_t = p_t0 + (C::PBUFS == 2 ? half * 32 : 0);
+                const uint32_t p_t = p_t0 + half * 32;
                 const uint64_t bd = v_desc0 + uint64_t((stage * C::V_TILE + half * (BS * C::V_ROW)) >> 4);
 #pragma unroll
-                for (int k = 0; k < (QA_ABL_PV > 0 ? QA_ABL_PV : BS / KEYS_PER_PV); ++k) {
+                for (int k = 0; k < BS / KEYS_PER_PV; ++k) {
                     const uint64_t bk = bd + uint64_t((k * KEYS_PER_PV * C::V_ROW) >> 4);
                     if constexpr (!C::V16) {
                         umma_f8_ts(o_t, p_t + k * 8, bk, idesc_pv, (acc || k > 0) ? 1u : 0u);
@@ -676,20 +539,14 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         }
     } else {
         // =============================================================== softmax / correction / epilogue
-        if constexpr (C::REBALANCE) reg_alloc<C::REG_SOFTMAX>();
-        constexpr int NH = C::NH, CW = C::CW;
-        const int t = warp / (4 * NH);                 // query tile of this warpgroup (pair)
-        const int hf = (warp >> 2) % NH;               // which CW-column share of every step this thread owns
+        if constexpr (C::REBALANCE) reg_alloc<kRegSoftmax>();
+        const int t = warp / 4;                        // query tile of this warpgroup
         const int row = ((warp & 3) << 5) | lane;      // row inside the tile == TMEM lane
         const uint32_t lane_base = uint32_t((warp & 3) * 32) << 16;
-        const uint32_t s_addr = tmem + lane_base + C::TM_S + t * 128 + hf * CW;
-        // a thread's share of a P buffer: CW keys = CW / 2 columns of 16-bit P, CW / 4 columns of e4m3 P
-        const uint32_t p_base = tmem + lane_base + C::TM_P + t * 128 + hf * (C::V16 ? CW / 2 : CW / 4);
-        // the NH threads of a row meet at a named barrier of their own (ids 1 .. 8) and swap values through shared memory
-        const uint32_t pair_bar = 1 + t * 4 + (warp & 3);
-        float* xchg = reinterpret_cast<float*>(smem + C::SMEM_XCHG) + (t * 2) * 128 + row;  // [t][share][row]
-        const uint32_t o_addr = tmem + lane_base + C::TM_O + (NQ == 2 ? t * 128 : 0);
-        const uint32_t l_addr = tmem + lane_base + C::TM_L + t * 128;
+        const uint32_t s_addr = lane_base + C::TM_S + t * 128;
+        const uint32_t p_base = lane_base + C::TM_P + t * 128;
+        const uint32_t o_addr = lane_base + C::TM_O + (NQ == 2 ? t * 128 : 0);
+        const uint32_t l_addr = lane_base + C::TM_L + t * 128;
         const int row_g = m0 + t * BM + row;
 
         float c;  // multiplier taking raw fp8 dot products to the base-2 softmax domain
@@ -711,8 +568,8 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         // only after P V of the tile's second step, i.e. after every softmax thread has published that step's P.
         int sk_slot = 0;
         uint32_t sk_phase = 0;
-        const uint32_t sk_base = smem_u32(smem + C::SMEM_SK) + uint32_t(hf * CW * 4);
-        auto kscale = [&](const int j, float (&s)[C::CW]) {
+        const uint32_t sk_base = smem_u32(smem + C::SMEM_SK);
+        auto kscale = [&](const int j, float (&s)[BS]) {
             if constexpr (TOKEN) {
                 if ((j & 1) == 0) {
                     if (j > 0 && ++sk_slot == C::STAGES) sk_slot = 0, sk_phase ^= 1;
@@ -720,7 +577,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
                 }
                 const uint32_t sk_addr = sk_base + uint32_t(sk_slot * (BN * 4) + (j & 1) * (BS * 4));
 #pragma unroll
-                for (int i = 0; i < CW; i += 4) {
+                for (int i = 0; i < BS; i += 4) {
                     const float4 k4 = lds_f32x4(sk_addr + i * 4);
                     const float2 a = __fmul2_rn(make_float2(s[i], s[i + 1]), make_float2(k4.x, k4.y));
                     const float2 bq = __fmul2_rn(make_float2(s[i + 2], s[i + 3]), make_float2(k4.z, k4.w));
@@ -731,21 +588,21 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         // causal / ragged mask of step j.  Only the trailing steps of a tile can need it (the ragged tail is the last
         // step, the causal diagonal the last two), so it is instantiated in the tail loop only: the main loop below
         // carries no mask code at all and stays a compact straight line for the instruction cache.
-        auto mask = [&](const int j, float (&s)[C::CW]) {
-            const int col0 = j * BS + hf * CW;
-            const bool tail = col0 + CW > p.Skv;
-            const bool diag = CAUSAL && (col0 + CW - 1 > m0 + t * BM);
+        auto mask = [&](const int j, float (&s)[BS]) {
+            const int col0 = j * BS;
+            const bool tail = col0 + BS > p.Skv;
+            const bool diag = CAUSAL && (col0 + BS - 1 > m0 + t * BM);
             if (tail || diag) {
                 const int lim = CAUSAL ? min(p.Skv - 1, row_g) : (p.Skv - 1);  // last visible column
 #pragma unroll
-                for (int i = 0; i < CW; ++i)
+                for (int i = 0; i < BS; ++i)
                     if (col0 + i > lim) s[i] = -INFINITY;
             }
         };
         // first step whose scores need the mask (every later one does too)
         const int j_mask = CAUSAL ? min(p.Skv / BS, (m0 + t * BM) / BS) : p.Skv / BS;
         // row maximum of sixteen columns folded into two running maxima (two chains per call site -> four in flight)
-        auto max16 = [&](const float (&s)[C::CW], int q, float& ma, float& mb) {
+        auto max16 = [&](const float (&s)[BS], int q, float& ma, float& mb) {
 #pragma unroll
             for (int i = 16 * q; i < 16 * q + 16; i += 4) {
                 ma = fmaxf(ma, fmaxf(s[i], s[i + 1]));
@@ -753,9 +610,9 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
             }
         };
         // rare: the running maximum of some row of this warp grew by more than 2^TAU -> rescale O (rolled: cold code)
-        auto rescale_o = [&](const float alpha) {  // (the NH threads of a row take D / NH columns each)
+        auto rescale_o = [&](const float alpha) {
 #pragma unroll 1
-            for (int cc = hf * (D / NH); cc < (hf + 1) * (D / NH); cc += 32) {
+            for (int cc = 0; cc < D; cc += 32) {
                 float o[32];
                 tmem_ld_x32(o_addr + cc, o);
                 tmem_ld_wait();
@@ -764,11 +621,9 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
                 tmem_st_x32(o_addr + cc, o);
             }
             if constexpr (C::MMASUM) {  // the row sum lives beside O and is rescaled with it
-                if (hf == 0) {
-                    float lv = tmem_ld_x1(l_addr);
-                    tmem_ld_wait();
-                    tmem_st_x1(l_addr, lv * alpha);
-                }
+                float lv = tmem_ld_x1(l_addr);
+                tmem_ld_wait();
+                tmem_st_x1(l_addr, lv * alpha);
             }
             tmem_st_wait();
         };
@@ -779,26 +634,24 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         // exponentials; it returns that maximum.  The code between the few waits is straight-line on purpose: every
         // branch is a scheduling barrier at which the exp pipeline of this warp drains.
         //   MASKED (compile time): S_{j+1} may need the causal / ragged mask;  `last`: there is no S_{j+1}.
-        constexpr int NQD = CW / 4;             // quads of columns per thread and step (16, or 8 with two threads per row)
-        constexpr int LOADQ = QA_LOADQ / NH;    // quad index (of NQD) before which the load of S_{j+1} is issued
-        static_assert(QA_LOADQ >= 2 && QA_LOADQ <= 12 && QA_LOADQ % 2 == 0, "LOADQ");
         //   `need` (warp-uniform): some row of the warp has outgrown its stale maximum, as decided near the END of the
         //   previous step (see below) - so the common case enters the exponentials with nothing to wait for.
-        auto step = [&](const int j, float (&s)[C::CW], float (&s_next)[C::CW], const float mx, bool& need, auto mask_tag,
+        auto step = [&](const int j, float (&s)[BS], float (&s_next)[BS], const float mx, bool& need, auto mask_tag,
                         const bool last) -> float {
             constexpr bool MASKED = decltype(mask_tag)::value;
+            // The schedule of the step, in quads of exponentials (four columns each, NQD per step).  Each constant was
+            // re-measured on the final kernel against its neighbours; none of those won on C2, C3 and D = 64 at once
+            // (profiles/r02_tune_ab.txt).
+            constexpr int NQD = BS / 4;
+            constexpr int PUBQ = 2;     // P_{j-1} (stored at the end of step j-1) is published after this many quads
+            constexpr int LOADQ = 8;    // S_{j+1} is pulled into registers after this many quads
+            constexpr int LDWAITQ = 4;  // quads between the TMEM load of S_{j+1} and the wait for it
+            constexpr int DECIDEQ = 1;  // quads left when the rescale decision for the next step is taken
             QA_STAMP(t, j, 0);
             bool p_prev_pending = j > 0;  // P_{j-1} is stored but not yet published (see below)
             // lazy rescale: keep the stale max while the true max has grown by < 2^TAU
             if (__builtin_expect(need, 0)) {
-                float m_new = fmaxf(m_used, mx);
-                if constexpr (NH == 2) {
-                    // the row's other thread holds the maximum of the other columns: swap through shared memory.  (The
-                    // slot is rewritten at the earliest on the next rescale, and a vote barrier lies in between.)
-                    xchg[hf * 128] = mx;
-                    named_bar_sync(pair_bar, 64);
-                    m_new = fmaxf(m_new, xchg[(hf ^ 1) * 128]);
-                }
+                const float m_new = fmaxf(m_used, mx);
                 const float alpha = ex2_approx((m_used - m_new) * c);  // 0 on the first step
                 m_used = m_new;
                 if constexpr (!C::MMASUM) la.x *= alpha, la.y *= alpha, lb.x *= alpha, lb.y *= alpha;
@@ -807,7 +660,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
                     // even start before P_{j-1} is published
                     tmem_st_wait();
                     tc_fence_before();
-                    softmax_arrive(&bars->p_full[t][(j - 1) & 1]);
+                    mbar_arrive(&bars->p_full[t][(j - 1) & 1]);
                     p_prev_pending = false;
                     // (one barrier per step parity: PV_{j-3}, the previous phase of this barrier, is known to be
                     // complete because S_j has been seen, so the parity test cannot alias)
@@ -822,25 +675,13 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
 
             // p' for one pair of columns; a compile-time subset of the pairs avoids MUFU
             auto exp_pair = [&](int i) -> float2 {
-                if (QA_ABL_EXP > 0 && i >= QA_ABL_EXP) return make_float2(s[2 * i], s[2 * i + 1]);
                 const float2 x = __ffma2_rn(make_float2(s[2 * i], s[2 * i + 1]), c2, neg2);
                 if (pair_uses_poly(i, C::POLY_NUM)) return exp2_poly<C::POLY_DEG>(x);
                 return make_float2(ex2_approx(x.x), ex2_approx(x.y));
             };
-            uint32_t pw[C::V16 ? CW / 2 : CW / 4], pw_lo[C::PMODE == QA_P_E4M3_HILO ? CW / 4 : 1];
+            uint32_t pw[C::V16 ? BS / 2 : BS / 4], pw_lo[C::PMODE == QA_P_E4M3_HILO ? BS / 4 : 1];
             // four columns -> P words (and, unless the tensor core sums the rows of P, the running row sum)
             auto exp_quad = [&](int i) {
-                if constexpr (C::H2POLY) {
-                    // each pair goes to e4m3 either from the half-precision polynomial or from two MUFU.EX2
-                    auto bytes2 = [&](int pr) -> uint16_t {
-                        const float2 x = __ffma2_rn(make_float2(s[2 * pr], s[2 * pr + 1]), c2, neg2);
-                        if (pair_uses_poly(pr, C::POLY_NUM)) return cvt_e4m3x2_from_h2(exp2_pair_h2(x));
-                        return cvt_e4m3x2_u16(ex2_approx(x.x), ex2_approx(x.y));
-                    };
-                    const uint16_t lo = bytes2(2 * i), hi = bytes2(2 * i + 1);
-                    pw[i] = join_u16(lo, hi);
-                    return;
-                }
                 const float2 p01 = exp_pair(2 * i), p23 = exp_pair(2 * i + 1);
                 if constexpr (!C::MMASUM) {
                     la = __fadd2_rn(la, p01);
@@ -859,152 +700,117 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
                 }
             };
 
-            constexpr int PUBQ = (QA_PUBQ / NH) > 0 ? QA_PUBQ / NH : 1, LDW = (QA_LDWAITQ / NH) > 0 ? QA_LDWAITQ / NH : 1;
-            constexpr int PROBEQ = QA_PROBEQ / NH;
-            static_assert(PUBQ >= 1 && PUBQ <= LOADQ - PROBEQ && LDW >= 1, "quad schedule");
 #pragma unroll
             for (int i = 0; i < PUBQ; ++i) exp_quad(i);
             if (p_prev_pending) {  // P_{j-1} was stored at the end of the previous step: publish it now
                 tmem_st_wait();
                 tc_fence_before();
-                softmax_arrive(&bars->p_full[t][(j - 1) & 1]);
+                mbar_arrive(&bars->p_full[t][(j - 1) & 1]);
             }
 #pragma unroll
-            for (int i = PUBQ; i < LOADQ - PROBEQ; ++i) exp_quad(i);
+            for (int i = PUBQ; i < LOADQ; ++i) exp_quad(i);
             float ma = -INFINITY, mb = -INFINITY;
             if (!last) {
                 // S_{j+1} was issued by the tensor core when this thread released S_j, about one step ago
-                bool s_ready = false;
-                if constexpr (PROBEQ > 0) {
-                    s_ready = mbar_test_wait(&bars->s_full[t], (j + 1) & 1);
-#pragma unroll
-                    for (int i = LOADQ - PROBEQ; i < LOADQ; ++i) exp_quad(i);
-                }
                 QA_STAMP(t, j, 5);
-                if (!s_ready) mbar_wait(&bars->s_full[t], (j + 1) & 1);
+                mbar_wait(&bars->s_full[t], (j + 1) & 1);
                 tc_fence_after();
-                if constexpr (NH == 1) tmem_ld_f64(s_addr, s_next);
-                else tmem_ld_x32(s_addr, s_next);
+                tmem_ld_f64(s_addr, s_next);
                 QA_STAMP(t, j, 2);
 #pragma unroll
-                for (int i = LOADQ; i < LOADQ + LDW; ++i) exp_quad(i);
+                for (int i = LOADQ; i < LOADQ + LDWAITQ; ++i) exp_quad(i);
                 tmem_ld_wait();
                 tc_fence_before();
-                softmax_arrive(&bars->s_free[t]);  // the score buffer may be overwritten by QK_{j+2}
+                mbar_arrive(&bars->s_free[t]);  // the score buffer may be overwritten by QK_{j+2}
                 kscale(j + 1, s_next);
                 if constexpr (MASKED) mask(j + 1, s_next);
                 QA_STAMP(t, j, 3);
-                // the row maximum of S_{j+1} is spread over the remaining quads but the last QA_DECIDEQ, four 16-column
+                // the row maximum of S_{j+1} is spread over the remaining quads but the last DECIDEQ, four 16-column
                 // pieces in all; the rescale decision for step j + 1 (a warp vote) is taken before those last quads, whose
                 // exponentials hide its latency
-                constexpr int DECQ = QA_DECIDEQ;
-                constexpr int REST = NQD - LDW - LOADQ - DECQ;  // quads carrying a piece of the maximum
-                static_assert(REST >= 1, "LOADQ / QA_DECIDEQ leave no room for the row maximum");
-                constexpr int NPIECE = CW / 16;               // 16-column pieces of the row maximum
+                constexpr int REST = NQD - LDWAITQ - LOADQ - DECIDEQ;  // quads carrying a piece of the maximum
+                static_assert(PUBQ <= LOADQ && REST >= 1, "quad schedule");
+                constexpr int NPIECE = BS / 16;                  // 16-column pieces of the row maximum
                 constexpr int PER = (NPIECE + REST - 1) / REST;  // pieces per quad
 #pragma unroll
-                for (int i = LOADQ + LDW; i < NQD - DECQ; ++i) {
+                for (int i = LOADQ + LDWAITQ; i < NQD - DECIDEQ; ++i) {
                     exp_quad(i);
 #pragma unroll
                     for (int q = 0; q < PER; ++q) {
-                        const int piece = (i - LOADQ - LDW) * PER + q;
+                        const int piece = (i - LOADQ - LDWAITQ) * PER + q;
                         if (piece < NPIECE) max16(s_next, piece, ma, mb);
                     }
                 }
-                if constexpr (NH == 1) {
-                    need = __any_sync(0xffffffffu, (fmaxf(ma, mb) - m_used) * c > C::TAU);
-                } else {
-                    // both threads of a row must take the rescale path together: an OR over the 64 threads of the pair
-                    need = bar_red_or(pair_bar, 64, (fmaxf(ma, mb) - m_used) * c > C::TAU);
-                }
+                need = __any_sync(0xffffffffu, (fmaxf(ma, mb) - m_used) * c > C::TAU);
 #pragma unroll
-                for (int i = NQD - DECQ; i < NQD; ++i) exp_quad(i);
+                for (int i = NQD - DECIDEQ; i < NQD; ++i) exp_quad(i);
             } else {
                 need = false;
 #pragma unroll
-                for (int i = LOADQ - PROBEQ; i < NQD; ++i) exp_quad(i);
-                // P buffer reuse (two buffers): PV_{j-2} must have drained it.  Seeing S_{j+1} (issued after PV_{j-2},
-                // in-order tensor pipe) proves that in every other step; the last one waits for PV_{j-1} explicitly.
-                if constexpr (C::PBUFS == 2) {
-                    if (j >= 2) mbar_wait(&bars->pv_done[t][(j - 1) & 1], ((j - 1) >> 1) & 1);
-                }
+                for (int i = LOADQ; i < NQD; ++i) exp_quad(i);
+                // P buffer reuse: PV_{j-2} must have drained it.  Seeing S_{j+1} (issued after PV_{j-2}, in-order
+                // tensor pipe) proves that in every other step; the last one waits for PV_{j-1} explicitly.
+                if (j >= 2) mbar_wait(&bars->pv_done[t][(j - 1) & 1], ((j - 1) >> 1) & 1);
             }
-            if constexpr (QA_SYNCCHECK != 0 && C::PBUFS == 2) {
+            if constexpr (QA_SYNCCHECK != 0) {
                 if (j >= 1 && !last) mbar_wait(&bars->pv_done[t][(j - 1) & 1], ((j - 1) >> 1) & 1);
             }
-            if constexpr (C::PBUFS == 1) {
-                // one P buffer: PV_{j-1} must have read P_{j-1} out of it.  It was published PUBQ quads into this
-                // step and the tensor pipe has had the whole step for it, so this wait is normally already satisfied.
-                if (j >= 1) {
-                    mbar_wait(&bars->pv_done[t][(j - 1) & 1], ((j - 1) >> 1) & 1);
-                    tc_fence_after();
-                }
-            }
-            const uint32_t p_addr = p_base + (C::PBUFS == 2 ? (j & 1) * 32 : 0);
+            // P_j goes to buffer j & 1 of the tile: 64 keys = 32 columns of 16-bit P or 16 columns of e4m3 P
+            const uint32_t p_addr = p_base + (j & 1) * 32;
             if constexpr (C::PMODE == QA_P_E4M3) {
-                tmem_st_words<CW / 4>(p_addr, pw);
+                tmem_st_words<BS / 4>(p_addr, pw);
             } else if constexpr (C::PMODE == QA_P_E4M3_HILO) {
-                tmem_st_words<CW / 4>(p_addr, pw);
-                tmem_st_words<CW / 4>(p_addr + C::TM_P_LO, pw_lo);
+                tmem_st_words<BS / 4>(p_addr, pw);
+                tmem_st_words<BS / 4>(p_addr + C::TM_P_LO, pw_lo);
             } else {
-                tmem_st_words<CW / 2>(p_addr, pw);
+                tmem_st_words<BS / 2>(p_addr, pw);
             }
             if (last) {  // nothing left to hide the store behind
                 tmem_st_wait();
                 tc_fence_before();
-                softmax_arrive(&bars->p_full[t][j & 1]);
+                mbar_arrive(&bars->p_full[t][j & 1]);
             }
             QA_STAMP(t, j, 4);
             return fmaxf(ma, mb);
         };
 
-#ifdef QA_STAGGER
-        if (t == 1) {  // start the second tile's softmax out of phase with the first
-            const long long t_go = clock64() + QA_STAGGER;
-            while (clock64() < t_go) {
-            }
-        }
-#endif
         if constexpr (C::QTMEM) {
             // this thread's query row -> tensor memory (lane = row, D bytes = D / 4 columns), straight from global
             // memory: the A operand of every Q K^T MMA of the tile
-            if (hf == 0) {
-                const uint8_t* qrow = p.q + (long long)b * p.q_sb + (long long)h * p.q_sh +
-                                      (long long)min(row_g, p.Sq - 1) * p.q_sr;
-                const uint32_t q_addr = tmem + lane_base + C::TM_Q + t * 128;
-                constexpr int NW = (D / 4 < 32) ? D / 4 : 32;  // words per tcgen05.st
+            const uint8_t* qrow = p.q + (long long)b * p.q_sb + (long long)h * p.q_sh +
+                                  (long long)min(row_g, p.Sq - 1) * p.q_sr;
+            const uint32_t q_addr = lane_base + C::TM_Q + t * 128;
+            constexpr int NW = (D / 4 < 32) ? D / 4 : 32;  // words per tcgen05.st
 #pragma unroll
-                for (int c0 = 0; c0 < D / 4; c0 += NW) {
-                    uint32_t w[NW];
+            for (int c0 = 0; c0 < D / 4; c0 += NW) {
+                uint32_t w[NW];
 #pragma unroll
-                    for (int i = 0; i < NW; i += 4) {
-                        const uint4 v = __ldg(reinterpret_cast<const uint4*>(qrow + (c0 + i) * 4));
-                        w[i] = v.x, w[i + 1] = v.y, w[i + 2] = v.z, w[i + 3] = v.w;
-                    }
-                    tmem_st_words<NW>(q_addr + c0, w);
+                for (int i = 0; i < NW; i += 4) {
+                    const uint4 v = __ldg(reinterpret_cast<const uint4*>(qrow + (c0 + i) * 4));
+                    w[i] = v.x, w[i + 1] = v.y, w[i + 2] = v.z, w[i + 3] = v.w;
                 }
-                tmem_st_wait();
-                tc_fence_before();
-                softmax_arrive(&bars->q_full[t]);
+                tmem_st_words<NW>(q_addr + c0, w);
             }
+            tmem_st_wait();
+            tc_fence_before();
+            mbar_arrive(&bars->q_full[t]);
         }
-        float s_a[CW], s_b[CW];
+        float s_a[BS], s_b[BS];
         float mx;
         QA_STAMP(t, 78, 1);
         {   // S_0
             mbar_wait(&bars->s_full[t], 0);
             QA_STAMP(t, 78, 2);
             tc_fence_after();
-            if constexpr (NH == 1) tmem_ld_f64(s_addr, s_a);
-            else tmem_ld_x32(s_addr, s_a);
+            tmem_ld_f64(s_addr, s_a);
             tmem_ld_wait();
             tc_fence_before();
-            softmax_arrive(&bars->s_free[t]);
+            mbar_arrive(&bars->s_free[t]);
             kscale(0, s_a);
             mask(0, s_a);
             float ma = -INFINITY, mb = -INFINITY;
 #pragma unroll
-            for (int q = 0; q < CW / 16; ++q) max16(s_a, q, ma, mb);
+            for (int q = 0; q < BS / 16; ++q) max16(s_a, q, ma, mb);
             mx = fmaxf(ma, mb);
         }
         {
@@ -1026,19 +832,13 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
             for (; j < my_steps; ++j) {
                 mx = step(j, s_a, s_b, mx, need, true_type{}, j + 1 == my_steps);
 #pragma unroll
-                for (int i = 0; i < CW; ++i) s_a[i] = s_b[i];
+                for (int i = 0; i < BS; ++i) s_a[i] = s_b[i];
             }
         }
         float l = (la.x + la.y) + (lb.x + lb.y);
-        if constexpr (NH == 2 && !C::MMASUM) {  // the row sum is the sum of the two threads' shares
-            named_bar_sync(pair_bar, 64);  // (the other thread may still be reading a maximum from the slot)
-            xchg[hf * 128] = l;
-            named_bar_sync(pair_bar, 64);
-            l += xchg[(hf ^ 1) * 128];
-        }
         QA_STAMP(t, 78, 3);
 
-        // ---------------------------------------------------------------- epilogue: O / l -> 16 bit -> smem -> TMA
+        // ---------------------------------------------------------------- epilogue: O / l -> 16 bit -> global memory
         mbar_wait(&bars->o_full[t], 0);
         tc_fence_after();
         QA_STAMP(t, 78, 4);
@@ -1048,15 +848,12 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         }
         const float sv = C::V16 ? 1.f : p.scale_v[bhkv];
         const float inv = __fdividef(sv, l);
-#if QA_DIRECT_STORE
         // A thread owns a whole output row (D * 2 contiguous bytes): it writes it straight from its registers, one
         // 32-byte sector per store.  Nothing to stage, fence or wait for - the CTA is free to retire as soon as the
-        // stores are issued, where the shared-memory + TMA route kept it alive until the bulk store had read the tile.
+        // stores are issued, where a shared-memory + TMA route would keep it alive until the bulk store had read the tile.
         uint8_t* o_row = static_cast<uint8_t*>(p.out) + (size_t(bh) * p.Sq + min(row_g, p.Sq - 1)) * (D * 2);
-        // (with NH threads per row each writes its D / NH columns: still whole 32-byte sectors)
 #pragma unroll
-        for (int c0 = 0; c0 < D / NH; c0 += 32) {
-            const int cc = hf * (D / NH) + c0;
+        for (int cc = 0; cc < D; cc += 32) {
             float o[32];
             tmem_ld_x32(o_addr + cc, o);
             tmem_ld_wait();
@@ -1071,53 +868,21 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
                 st_global_32B(o_row + cc * 2 + 32, w + 8);
             }
         }
-        if (p.lse != nullptr && row_g < p.Sq && hf == 0)
-            p.lse[size_t(bh) * p.Sq + row_g] = (m_used * c + (__log2f(l) - C::KOFF)) * 0.6931471805599453f;
-#else
-        uint8_t* o_smem = smem + C::SMEM_O + t * C::O_TILE;
-#pragma unroll
-        for (int cc = 0; cc < D; cc += 32) {
-            float o[32];
-            tmem_ld_x32(o_addr + cc, o);
-            tmem_ld_wait();
-            uint32_t w[16];
-#pragma unroll
-            for (int i = 0; i < 16; ++i) {
-                const float a = o[2 * i] * inv, bb = o[2 * i + 1] * inv;
-                w[i] = p.out_fp16 ? pack_f16x2(a, bb) : pack_bf16x2(a, bb);
-            }
-            // 64 output columns (128 bytes) per box row, 128B-swizzled so the TMA store un-swizzles it
-            uint8_t* box = o_smem + (cc >> 6) * (BM * 128) + row * 128;
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-                const int chunk = ((cc & 63) >> 3) + q;
-                *reinterpret_cast<uint4*>(box + ((chunk ^ (row & 7)) << 4)) =
-                    make_uint4(w[4 * q], w[4 * q + 1], w[4 * q + 2], w[4 * q + 3]);
-            }
-        }
         if (p.lse != nullptr && row_g < p.Sq)
             p.lse[size_t(bh) * p.Sq + row_g] = (m_used * c + (__log2f(l) - C::KOFF)) * 0.6931471805599453f;
-        fence_proxy_async_smem();
-        named_bar_sync(1 + t, 128);
-        if ((warp & 3) == 0 && lane == 0 && m0 + t * BM < p.Sq) {
-            for (int x = 0; x < C::O_BOXES; ++x) tma_store_3d(&tmO, o_smem + x * (BM * 128), x * 64, m0 + t * BM, bh);
-            tma_store_commit();
-            tma_store_wait_read<0>();  // the CTA only has to keep its shared memory alive until it has been read
-        }
-#endif
         QA_STAMP(t, 78, 5);
     }
 
     tc_fence_before();
     __syncthreads();
-    if (warp == 0) tmem_dealloc(tmem, C::TMEM_COLS);
+    if (warp == 0) tmem_dealloc(0, kTmemCols);
     QA_STAMP(warp >> 2, 78, 6);
 }
 
 // ------------------------------------------------------------------------------------------------ host side
 template <class C, bool CAUSAL, bool TOKEN>
 static int launch_cfg(const AttnArgs& a, cudaStream_t stream, int* launches) {
-    CUtensorMap tmQ, tmK, tmV, tmO;
+    CUtensorMap tmQ, tmK, tmV;
     const CUtensorMapSwizzle qk_swz = C::QK_ROW == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
     const CUtensorMapSwizzle v_swz = C::V_ROW == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
     const uint64_t D = C::D;
@@ -1137,10 +902,6 @@ static int launch_cfg(const AttnArgs& a, cudaStream_t stream, int* launches) {
         ok &= make_tmap_4d(&tmV, dt, a.v, D, a.Skv, a.Hkv, a.B, a.vs[2] * C::VB, a.vs[1] * C::VB, a.vs[0] * C::VB,
                            C::V_ROW / C::VB, BN, v_swz);
     }
-    const CUtensorMapDataType odt =
-        a.out_dtype == QA_DT_FP16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
-    ok &= make_tmap_3d(&tmO, odt, 2, a.out, D, a.Sq, uint64_t(a.B) * a.Hq, D * 2, D * 2 * a.Sq, 64, BM,
-                       CU_TENSOR_MAP_SWIZZLE_128B);
     if (!ok) return set_error(QA_ERR_DEVICE, "cuTensorMapEncodeTiled failed or is unavailable (no CUDA driver?)");
 
     AttnParams p;
@@ -1173,14 +934,10 @@ static int launch_cfg(const AttnArgs& a, cudaStream_t stream, int* launches) {
     if (!attr_done.has(dev)) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_TOTAL);
         if (e != cudaSuccess) return set_cuda_error("cudaFuncSetAttribute(max dynamic smem)", e);
-        if (C::CTAS_PER_SM > 1) {  // two CTAs per SM need the largest shared-memory carve-out
-            e = cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-            if (e != cudaSuccess) return set_cuda_error("cudaFuncSetAttribute(carve-out)", e);
-        }
         attr_done.add(dev);
     }
     dim3 grid((a.Sq + BM * C::NQ - 1) / (BM * C::NQ), a.Hq, a.B);
-    cudaError_t e = launch_pdl(kern, grid, dim3(C::NTHREADS), size_t(C::SMEM_TOTAL), stream, tmQ, tmK, tmV, tmO, p);
+    cudaError_t e = launch_pdl(kern, grid, dim3(C::NTHREADS), size_t(C::SMEM_TOTAL), stream, tmQ, tmK, tmV, p);
     if (e == cudaSuccess) e = cudaGetLastError();
     if (e != cudaSuccess) return set_cuda_error("attn_fwd_kernel launch", e);
     *launches += 1;

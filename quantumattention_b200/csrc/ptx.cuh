@@ -142,21 +142,6 @@ __device__ __forceinline__ void bulk_load_1d(void* smem_dst, const void* gsrc, u
         : "r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(gsrc)), "r"(bytes), "r"(smem_u32(bar)), "l"(policy)
         : "memory");
 }
-__device__ __forceinline__ void tma_store_3d(const CUtensorMap* m, const void* smem_src, int c0, int c1, int c2) {
-    asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
-                 :
-                 : "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(smem_src)), "r"(c0), "r"(c1), "r"(c2)
-                 : "memory");
-}
-__device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void tma_store_wait_read() {
-    asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
-}
-template <int N>
-__device__ __forceinline__ void tma_store_wait_all() {
-    asm volatile("cp.async.bulk.wait_group %0;" ::"n"(N) : "memory");
-}
 
 
 // ----------------------------------------------------------------------------------------------- tcgen05 / TMEM
@@ -410,22 +395,6 @@ __device__ __forceinline__ uint32_t pack_e4m3x4(float a, float b, float c, float
     asm("mov.b32 %0, {%1, %2};" : "=r"(r) : "h"(lo), "h"(hi));
     return r;
 }
-// two halves (an f16x2 word) -> two e4m3 bytes
-__device__ __forceinline__ uint16_t cvt_e4m3x2_from_h2(uint32_t h2) {
-    uint16_t r;
-    asm("cvt.rn.satfinite.e4m3x2.f16x2 %0, %1;" : "=h"(r) : "r"(h2));
-    return r;
-}
-__device__ __forceinline__ uint16_t cvt_e4m3x2_u16(float lo, float hi) {
-    uint16_t r;
-    asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(r) : "f"(hi), "f"(lo));
-    return r;
-}
-__device__ __forceinline__ uint32_t join_u16(uint16_t lo, uint16_t hi) {
-    uint32_t r;
-    asm("mov.b32 %0, {%1, %2};" : "=r"(r) : "h"(lo), "h"(hi));
-    return r;
-}
 __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
     uint32_t r;
     asm("cvt.rn.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
@@ -444,26 +413,6 @@ __device__ __forceinline__ float2 e4m3x2_to_float2(uint32_t v) {
     return __half22float2(h);
 }
 
-// named barrier among a subset of warps
-__device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t nthreads) {
-    asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
-}
-
-// barrier with an OR reduction over the participating threads' predicates (all of them receive the result)
-__device__ __forceinline__ bool bar_red_or(uint32_t id, uint32_t nthreads, bool pred) {
-    uint32_t r;
-    asm volatile(
-        "{\n\t"
-        ".reg .pred pin, pout;\n\t"
-        "setp.ne.u32 pin, %1, 0;\n\t"
-        "bar.red.or.pred pout, %2, %3, pin;\n\t"
-        "selp.u32 %0, 1, 0, pout;\n\t"
-        "}\n"
-        : "=r"(r)
-        : "r"(uint32_t(pred)), "r"(id), "r"(nthreads)
-        : "memory");
-    return r != 0;
-}
 // N words (8 / 16 / 32) of a thread's registers -> N consecutive TMEM columns of its lane
 template <int N>
 __device__ __forceinline__ void tmem_st_words(uint32_t taddr, const uint32_t* r);
