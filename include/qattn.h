@@ -43,10 +43,7 @@ extern "C" {
                                     that shards one sequence over several GPUs take the MAX of the per-shard scales
                                     (scale is monotone in amax) and obtain the bytes the unsharded call would produce */
 
-#define QA_SCALE_HEAD_RELOAD 5    /* qa_quantize_fp8 only: QA_SCALE_HEAD results; heads too long for the single-pass ring take
-                                    the single-pass RELOAD variant (each slab loaded twice, the second time from L2: 3 bytes
-                                    of DRAM traffic per element instead of the two passes' 5) where its geometry allows.
-                                    Measured slower than the two passes on B200 (see csrc/quantize.cu), hence opt-in */
+#define QA_SCALE_HEAD_RELOAD 5    /* accepted for ABI 6 compatibility; same as QA_SCALE_HEAD */
 
 #define QA_WS_PERSISTENT 0x100    /* qa_quantize_fp8, OR-ed into scale_mode: amax_ws was zero-filled ONCE by the caller
                                     when it was allocated and has since been written only by this library (calls of any

@@ -96,9 +96,8 @@ static int quantize_call(int n_tensors, const void* const* x, int x_dtype, const
     const bool ws_persistent = (scale_mode & QA_WS_PERSISTENT) != 0;
     scale_mode &= ~QA_WS_PERSISTENT;
     const bool two_pass = scale_mode == QA_SCALE_HEAD_TWO_PASS;
-    const bool reload = scale_mode == QA_SCALE_HEAD_RELOAD;
     const bool given = scale_mode == QA_SCALE_HEAD_GIVEN, amax_only = scale_mode == QA_SCALE_HEAD_AMAX_ONLY;
-    if (two_pass || given || amax_only || reload) scale_mode = QA_SCALE_HEAD;
+    if (two_pass || given || amax_only || scale_mode == QA_SCALE_HEAD_RELOAD) scale_mode = QA_SCALE_HEAD;
     if (scale_mode != QA_SCALE_HEAD && scale_mode != QA_SCALE_TOKEN)
         return set_error(QA_ERR_INVALID, "Unsupported scaling_method code: %d", scale_mode);
     if (D != 64 && D != 128 && D != 256) return set_error(QA_ERR_INVALID, "Unsupported head dimension: %d", D);
@@ -126,7 +125,6 @@ static int quantize_call(int n_tensors, const void* const* x, int x_dtype, const
     a.ctl = reinterpret_cast<unsigned int*>(amax_ws);
     a.cells = amax_ws ? amax_ws + 8 : nullptr;
     a.force_two_pass = two_pass ? 1 : 0;
-    a.force_reload = reload ? 1 : 0;
     a.given_scale = given ? 1 : 0;
     a.amax_only = amax_only ? 1 : 0;
     a.ws_persistent = ws_persistent ? 1 : 0;

@@ -64,20 +64,6 @@ __device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
         : "memory");
     return ok != 0;
 }
-// non-blocking probe (try_wait may suspend the thread for a hardware-defined time; test_wait never does)
-__device__ __forceinline__ bool mbar_test_wait(uint64_t* bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t"
-        ".reg .pred P1;\n\t"
-        "mbarrier.test_wait.parity.shared::cta.b64 P1, [%1], %2;\n\t"
-        "selp.b32 %0, 1, 0, P1;\n\t"
-        "}\n"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
 #if QA_WATCHDOG
     // try_wait suspends in hardware for a bounded time per call, so a few million polls is seconds of wall clock.

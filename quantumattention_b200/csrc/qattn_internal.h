@@ -80,7 +80,6 @@ struct QuantArgs {
     float* cells;       // workspace + 8: amax cells of the two-pass kernels, then the single-pass kernel's slots
     int rows_per_cta;
     int force_two_pass;
-    int force_reload;   // QA_SCALE_HEAD_RELOAD: long heads take the single-pass reload variant where its geometry allows
     int given_scale;  // QA_SCALE_HEAD_GIVEN: scale[] is an input
     int amax_only;    // QA_SCALE_HEAD_AMAX_ONLY: write scale[] only
     size_t ws_floats;

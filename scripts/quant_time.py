@@ -28,5 +28,5 @@ for name, (H, S, D, n) in {"C2": (24, 4608, 128, 2), "C3": (32, 8192, 128, 2), "
     torch.cuda.synchronize()
     ms = a.elapsed_time(b) / (4 * reps)
     by = n * H * S * D * 3
-    print(f"{name}: {ms * 1e3:7.1f} us  {by / ms / 1e6:6.0f} GB/s  launches/call {nl} reload={os.environ.get('QA_QUANT_RELOAD', '1')}", flush=True)
+    print(f"{name}: {ms * 1e3:7.1f} us  {by / ms / 1e6:6.0f} GB/s  launches/call {nl}", flush=True)
     del sets, g

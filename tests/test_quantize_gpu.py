@@ -155,21 +155,24 @@ def test_long_head_takes_two_pass_path():
 
 
 @pytest.mark.parametrize("shape,n_tensors", [((1, 2, 75600, 128), 3), ((1, 1, 60000, 256), 1), ((2, 1, 100001, 64), 2)])
-def test_long_heads_single_pass_reload_variant(shape, n_tensors):
-    """Heads that span 4 - 10 trips of the grid (the long-video shape: 591 slabs per head on 148 SMs) can take the
-    single-pass variant that loads every slab twice - amax pass from HBM, quantise pass from L2 - in ONE launch
-    (QA_SCALE_HEAD_RELOAD; opt-in, the two passes are faster on B200); bytes and scales identical to the oracle and to
-    the two-pass kernels, ragged lengths and several tensors included."""
+def test_long_heads_reload_mode_is_head_wise(shape, n_tensors):
+    """Heads that span 4 - 10 trips of the grid (the long-video shape: 591 slabs per head on 148 SMs), through the
+    default head-wise mode and through QA_SCALE_HEAD_RELOAD, which ABI 6 callers may still pass: both take the same
+    kernels, and their bytes and scales are identical to the oracle and to the two-pass kernels, ragged lengths and
+    several tensors included."""
     g = torch.Generator().manual_seed(shape[2])
     xs = [(torch.randn(shape, generator=g) * (1.0 + i)).to(torch.bfloat16) for i in range(n_tensors)]
     if n_tensors > 1:  # ragged: a shorter second tensor
         xs[1] = xs[1][:, :, : shape[2] - 777].contiguous()
     xc = [x.cuda() for x in xs]
     outs, scales = _native.quantize_fp8(xc, _native.QA_SCALE_HEAD_RELOAD)
-    assert _native.last_launch_count() == 1
+    n_reload = _native.last_launch_count()
+    outs1, scales1 = _native.quantize_fp8(xc, _native.QA_SCALE_HEAD)
+    assert _native.last_launch_count() == n_reload
     outs2, scales2 = _native.quantize_fp8(xc, _native.QA_SCALE_HEAD_TWO_PASS)
-    for x, o, sc, o2, sc2 in zip(xs, outs, scales, outs2, scales2):
+    for x, o, sc, o1, sc1, o2, sc2 in zip(xs, outs, scales, outs1, scales1, outs2, scales2):
         assert torch.equal(o.view(torch.uint8), o2.view(torch.uint8)) and torch.equal(sc, sc2)
+        assert torch.equal(o1.view(torch.uint8), o2.view(torch.uint8)) and torch.equal(sc1, sc2)
         b, s_ = oracle.quantize_fp8(x.float().numpy(), "head-wise")
         assert np.array_equal(sc.cpu().numpy(), s_) and np.array_equal(o.view(torch.uint8).cpu().numpy(), b)
     # back to back on the persistent workspace, other shapes in between
