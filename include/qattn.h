@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define QA_ABI_VERSION 6
+#define QA_ABI_VERSION 7
 
 /* element types */
 #define QA_DT_BF16 0
@@ -59,6 +59,12 @@ extern "C" {
 #define QA_P_E4M3_HILO 1 /* P -> e4m3 hi + e4m3 lo (two MMAs), V e4m3            (accurate FP8 path)             */
 #define QA_P_16BIT 2     /* P -> bf16/fp16, V unquantised 16-bit, kind::f16       (the reference's own numerics:  */
                          /*                                   src/quantum_attn/tk/attention.py:230,286,318)      */
+
+/* the `causal` argument of the attention entry points (0: no mask) */
+#define QA_CAUSAL_TOP_LEFT 1     /* row i sees keys j <= i: torch SDPA's is_causal (src/quantum_attn/tk/attention.py:252-263) */
+#define QA_CAUSAL_BOTTOM_RIGHT 2 /* row i sees keys j <= i + Skv - Sq; needs Sq <= Skv.  The last query row is aligned with
+                                    the last key: a block of queries that sits at the END of the keys it attends, as a
+                                    sequence shard does against the keys of the shards before it */
 
 /* error codes */
 #define QA_OK 0
@@ -121,7 +127,9 @@ int qa_quantize_fp8(int n_tensors, const void* const* x, int x_dtype, const int6
  *               weight sits up to TAU = 4 log2 units above the stale running maximum.  Merging partial results with
  *               it reproduces the one-launch result.
  *   sm_scale    softmax scale; pass 1/sqrt(D) for the reference's behaviour (src/quantum_attn/tk/attention.py:208-210)
- *   Hq % Hkv == 0 (GQA: kv head = q head / (Hq/Hkv)); D in {64, 128, 256}; causal mask is top-left aligned.
+ *   causal      0, QA_CAUSAL_TOP_LEFT (the reference's mask) or QA_CAUSAL_BOTTOM_RIGHT (Sq <= Skv); other values and
+ *               bottom-right with Sq > Skv return QA_ERR_INVALID
+ *   Hq % Hkv == 0 (GQA: kv head = q head / (Hq/Hkv)); D in {64, 128, 256}.
  */
 int qa_fp8_attn_fwd(const void* q8, const void* k8, const void* v, int v_dtype, const int64_t* q_strides,
                     const int64_t* k_strides, const int64_t* v_strides, const float* scale_q, const float* scale_k,
@@ -138,6 +146,7 @@ int qa_fp8_attn_fwd(const void* q8, const void* k8, const void* v, int v_dtype, 
  * waiting for the slowest CTA of the one before it: +12 % at 148 CTAs per group, profiles/r02_wave_probe.txt).
  * Q must be complete in stream order (it is local).  Only for transfers that need no SM (copy engines): a transfer
  * KERNEL could find every SM held by a polling CTA.  A flag that never arrives traps the kernel after ~4 s of polling.
+ * QA_CAUSAL_BOTTOM_RIGHT returns QA_ERR_UNSUPPORTED here.
  */
 int qa_fp8_attn_fwd_gated(const void* q8, const void* k8, const void* v, int v_dtype, const int64_t* q_strides,
                           const int64_t* k_strides, const int64_t* v_strides, const float* scale_q, const float* scale_k,
@@ -176,7 +185,7 @@ int qa_fp8_attn_func(const void* q, const void* k, const void* v, int dtype, con
  *   q, k, v     [B,Hq,Sq,D], [B,Hkv,Skv,D], [B,Hkv,Skv,D], all of `dtype` (QA_DT_BF16 / QA_DT_FP16), optional element
  *               strides (batch, head, row) as in qa_fp8_attn_fwd
  *   out         dense [B,Hq,Sq,D] of `dtype`;  lse as in qa_fp8_attn_fwd (NULL to skip)
- *   Hq % Hkv == 0; D in {64, 128, 256}; causal mask is top-left aligned.
+ *   Hq % Hkv == 0; D in {64, 128, 256}; causal as in qa_fp8_attn_fwd.
  */
 int qa_attn_fwd(const void* q, const void* k, const void* v, int dtype, const int64_t* q_strides,
                 const int64_t* k_strides, const int64_t* v_strides, void* out, float* lse, int B, int Hq, int Hkv, int Sq,

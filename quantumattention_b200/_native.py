@@ -19,7 +19,8 @@ QA_SCALE_HEAD, QA_SCALE_TOKEN, QA_SCALE_HEAD_TWO_PASS, QA_SCALE_HEAD_AMAX_ONLY, 
 QA_SCALE_HEAD_RELOAD = 5
 QA_WS_PERSISTENT = 0x100  # qa_quantize_fp8: the workspace was zeroed once and is reused (include/qattn.h)
 QA_P_E4M3, QA_P_E4M3_HILO, QA_P_16BIT = 0, 1, 2
-ABI_VERSION = 6
+QA_CAUSAL_TOP_LEFT, QA_CAUSAL_BOTTOM_RIGHT = 1, 2  # the `causal` argument of the attention entries (0: no mask)
+ABI_VERSION = 7
 
 EXPORTED_SYMBOLS = (
     "qa_abi_version",
@@ -296,10 +297,11 @@ def _f32c(t: Optional[torch.Tensor]):
 
 
 def fp8_attn_fwd(q8: torch.Tensor, k8: torch.Tensor, v: torch.Tensor, scale_q: torch.Tensor, scale_k: torch.Tensor,
-                 scale_v: Optional[torch.Tensor], *, scale_mode: int, is_causal: bool, sm_scale: float, p_mode: int,
+                 scale_v: Optional[torch.Tensor], *, scale_mode: int, is_causal, sm_scale: float, p_mode: int,
                  out_dtype: torch.dtype, return_lse: bool = False, out: Optional[torch.Tensor] = None, gate=None):
     """Launch the fused forward kernel.  q8/k8 e4m3 [B,H,S,D]; v e4m3 (+scale_v) or bf16/fp16.  Tensors whose last
-    dim is contiguous and whose strides are 16-byte multiples ([B,S,H,D]-held views) are read in place.  ``out``:
+    dim is contiguous and whose strides are 16-byte multiples ([B,S,H,D]-held views) are read in place.  ``is_causal``:
+    a bool (top-left mask) or QA_CAUSAL_BOTTOM_RIGHT (row i sees keys <= i + Skv - Sq; Sq <= Skv).  ``out``:
     optional dense [B,Hq,Sq,D] destination (e.g. a head range of a larger output).  ``gate``: optional
     (flags int32 tensor, heads_per_gate, flags_per_gate) - a gated launch (``qa_fp8_attn_fwd_gated``): the CTAs of kv
     head h read K / V only once flags[(h // heads_per_gate) * flags_per_gate : ... + flags_per_gate] are non-zero
@@ -332,7 +334,7 @@ def fp8_attn_fwd(q8: torch.Tensor, k8: torch.Tensor, v: torch.Tensor, scale_q: t
         common = (q8.data_ptr(), k8.data_ptr(), v.data_ptr(), _dt_code(v.dtype), qs, ks, vs, scale_q.data_ptr(),
                   scale_k.data_ptr(), scale_v.data_ptr() if scale_v is not None else None, scale_mode, out.data_ptr(),
                   _dt_code(out_dtype), lse.data_ptr() if lse is not None else None, B, Hq, Hkv, Sq, Skv, D,
-                  int(bool(is_causal)), float(sm_scale), p_mode)
+                  int(is_causal), float(sm_scale), p_mode)
         if gate is None:
             rc = lib.qa_fp8_attn_fwd(*common, stream)
         else:
@@ -416,10 +418,10 @@ def fp8_attn_func(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, *, scale_mo
     return res, quant
 
 
-def attn_fwd(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, *, is_causal: bool, sm_scale: float,
+def attn_fwd(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, *, is_causal, sm_scale: float,
              return_lse: bool = False):
     """Launch the fused forward kernel on 16-bit q, k, v (all bf16 or all fp16), [B,H,S,D] (strided views are read in
-    place when their strides are 16-byte multiples)."""
+    place when their strides are 16-byte multiples).  ``is_causal`` as in ``fp8_attn_fwd``."""
     lib = load()
     B, Hq, Sq, D = q.shape
     Hkv, Skv = k.shape[1], k.shape[2]
@@ -435,7 +437,7 @@ def attn_fwd(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, *, is_causal: bo
             ev0.record(tstream)
         rc = lib.qa_attn_fwd(q.data_ptr(), k.data_ptr(), v.data_ptr(), _dt_code(q.dtype), qs, ks, vs, out.data_ptr(),
                              lse.data_ptr() if lse is not None else None, B, Hq, Hkv, Sq, Skv, D,
-                             int(bool(is_causal)), float(sm_scale), _raw_stream(idx))
+                             int(is_causal), float(sm_scale), _raw_stream(idx))
         if attn_events is not None:
             ev1.record(tstream)
             attn_events.append((ev0, ev1))

@@ -53,6 +53,17 @@ static int take_strides(int64_t (&dst)[3], const int64_t* src, int B, int H, int
     return QA_OK;
 }
 
+// The `causal` argument of the attention entry points: 0, QA_CAUSAL_TOP_LEFT or QA_CAUSAL_BOTTOM_RIGHT (Sq <= Skv).
+static int check_causal(int causal, int Sq, int Skv) {
+    if (causal != 0 && causal != QA_CAUSAL_TOP_LEFT && causal != QA_CAUSAL_BOTTOM_RIGHT)
+        return set_error(QA_ERR_INVALID, "causal must be 0, QA_CAUSAL_TOP_LEFT (1) or QA_CAUSAL_BOTTOM_RIGHT (2), got %d",
+                         causal);
+    if (causal == QA_CAUSAL_BOTTOM_RIGHT && Sq > Skv)
+        return set_error(QA_ERR_INVALID,
+                         "QA_CAUSAL_BOTTOM_RIGHT needs Sq <= Skv (every row must see a key), got Sq=%d and Skv=%d", Sq, Skv);
+    return QA_OK;
+}
+
 }  // namespace qa
 
 using namespace qa;
@@ -153,6 +164,7 @@ static int fp8_attn_call(const void* q8, const void* k8, const void* v, int v_dt
         return set_error(QA_ERR_INVALID, "gated launch: heads_per_gate >= 1 and 1 <= flags_per_gate <= 64 expected");
     if (D != 64 && D != 128 && D != 256) return set_error(QA_ERR_INVALID, "Unsupported head dimension: %d", D);
     if (B < 1 || Hq < 1 || Hkv < 1 || Sq < 1 || Skv < 1) return set_error(QA_ERR_INVALID, "empty problem");
+    if (int rc = check_causal(causal, Sq, Skv)) return rc;
     if (Hq % Hkv != 0)
         return set_error(QA_ERR_INVALID, "Expect Hq to be a multiple of Hkv but got Hq=%d and Hkv=%d.", Hq, Hkv);
     if (Hq > 65535 || B > 65535) return set_error(QA_ERR_INVALID, "B or Hq exceeds the grid limit 65535");
@@ -184,7 +196,7 @@ static int fp8_attn_call(const void* q8, const void* k8, const void* v, int v_dt
     a.scale_q = scale_q, a.scale_k = scale_k, a.scale_v = scale_v;
     a.out = out, a.lse = lse;
     a.B = B, a.Hq = Hq, a.Hkv = Hkv, a.Sq = Sq, a.Skv = Skv, a.D = D;
-    a.causal = causal ? 1 : 0;
+    a.causal = causal;
     a.sm_scale = sm_scale;
     a.scale_mode = scale_mode;
     a.p_mode = p_mode;
@@ -202,6 +214,8 @@ int qa_fp8_attn_fwd_gated(const void* q8, const void* k8, const void* v, int v_d
                           const unsigned* kv_ready, int heads_per_gate, int flags_per_gate, void* stream) {
     g_launches = 0;
     if (!kv_ready) return set_error(QA_ERR_INVALID, "null pointer argument");
+    if (causal == QA_CAUSAL_BOTTOM_RIGHT)
+        return set_error(QA_ERR_UNSUPPORTED, "gated launch: QA_CAUSAL_BOTTOM_RIGHT is not supported");
     return fp8_attn_call(q8, k8, v, v_dtype, q_strides, k_strides, v_strides, scale_q, scale_k, scale_v, scale_mode, out,
                          out_dtype, lse, B, Hq, Hkv, Sq, Skv, D, causal, sm_scale, p_mode, stream, kv_ready,
                          heads_per_gate, flags_per_gate);
@@ -308,6 +322,7 @@ int qa_attn_fwd(const void* q, const void* k, const void* v, int dtype, const in
         return set_error(QA_ERR_INVALID, "Expected query, key, and value to have dtype fp16 or bf16 (code %d)", dtype);
     if (D != 64 && D != 128 && D != 256) return set_error(QA_ERR_INVALID, "Unsupported head dimension: %d", D);
     if (B < 1 || Hq < 1 || Hkv < 1 || Sq < 1 || Skv < 1) return set_error(QA_ERR_INVALID, "empty problem");
+    if (int rc = check_causal(causal, Sq, Skv)) return rc;
     if (Hq % Hkv != 0)
         return set_error(QA_ERR_INVALID, "Expect Hq to be a multiple of Hkv but got Hq=%d and Hkv=%d.", Hq, Hkv);
     if (Hq > 65535 || B > 65535) return set_error(QA_ERR_INVALID, "B or Hq exceeds the grid limit 65535");
@@ -325,7 +340,7 @@ int qa_attn_fwd(const void* q, const void* k, const void* v, int dtype, const in
     a.scale_q = a.scale_k = a.scale_v = nullptr;
     a.out = out, a.lse = lse;
     a.B = B, a.Hq = Hq, a.Hkv = Hkv, a.Sq = Sq, a.Skv = Skv, a.D = D;
-    a.causal = causal ? 1 : 0;
+    a.causal = causal;
     a.sm_scale = sm_scale;
     a.scale_mode = QA_SCALE_HEAD;
     a.p_mode = QA_P_16BIT;

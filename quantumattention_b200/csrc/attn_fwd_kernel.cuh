@@ -4,7 +4,8 @@
 //
 // What it replaces: `fwd_attend_ker` of the reference (src/quantum_attn/tk/attention.py:97-349) and its launcher
 // (:355-647).  Same function (dequant scale folded into the exp2 argument as in :204-210,248-250; top-left causal
-// mask as in :252-263; ragged tails via TMA zero fill + -inf columns as in :269-271), different machine:
+// mask as in :252-263, or shifted by a run-time diagonal offset for the bottom-right alignment of the C ABI; ragged
+// tails via TMA zero fill + -inf columns as in :269-271), different machine:
 //
 //   CTA = 2 query tiles of 128 rows, 12 warps (3 warpgroups; setmaxnreg moves registers to the softmax warps):
 //     warps 0-3  softmax + (rare) O rescale + epilogue of query tile 0   (thread r <-> TMEM lane r <-> query row r)
@@ -151,6 +152,7 @@ struct AttnParams {
     long long q_sb, q_sh, q_sr;
     int B, Hq, Hkv, Sq, Skv;
     int causal;
+    int off;  // causal diagonal offset (>= 0): row i sees keys j <= i + off (0: top-left, Skv - Sq: bottom-right)
     float sm_scale_log2;  // sm_scale * log2(e)
     int out_fp16;
     int qk_fp16;  // QK16 configs: element type of Q and K
@@ -233,9 +235,11 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
     const int mblk = CAUSAL ? (gridDim.x - 1 - blockIdx.x) : blockIdx.x;
     const int m0 = mblk * (BM * NQ);
     const int nst_all = (p.Skv + BS - 1) / BS;
-    // per-tile trip counts in 64-key steps: under a causal mask tile t stops at its own diagonal
-    const int nst0 = CAUSAL ? min(nst_all, m0 / BS + 2) : nst_all;
-    const int nst1 = CAUSAL ? min(nst_all, (m0 + BM) / BS + 2) : nst_all;
+    // per-tile trip counts in 64-key steps: under a causal mask tile t stops at the step holding its last row's last
+    // visible key, off + m0 + t * BM + BM - 1.  The producer (n_kv), the MMA warps and the softmax warps all take their
+    // counts from n_steps(): a count that differed between the roles would leave a barrier waiting for ever
+    const int nst0 = CAUSAL ? min(nst_all, (p.off + m0 + BM - 1) / BS + 1) : nst_all;
+    const int nst1 = CAUSAL ? min(nst_all, (p.off + m0 + 2 * BM - 1) / BS + 1) : nst_all;
     auto n_steps = [&](int t) { return t == 0 ? nst0 : nst1; };
     const int n_max = n_steps(NQ - 1);
     const int n_kv = (n_max + 1) >> 1;  // K/V tiles of 128 keys
@@ -548,6 +552,7 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         const uint32_t o_addr = lane_base + C::TM_O + (NQ == 2 ? t * 128 : 0);
         const uint32_t l_addr = lane_base + C::TM_L + t * 128;
         const int row_g = m0 + t * BM + row;
+        const int diag_t = CAUSAL ? p.off + m0 + t * BM : 0;  // last key the tile's first row sees (causal)
 
         float c;  // multiplier taking raw fp8 dot products to the base-2 softmax domain
         if constexpr (C::QK16) {
@@ -591,16 +596,16 @@ attn_fwd_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__
         auto mask = [&](const int j, float (&s)[BS]) {
             const int col0 = j * BS;
             const bool tail = col0 + BS > p.Skv;
-            const bool diag = CAUSAL && (col0 + BS - 1 > m0 + t * BM);
+            const bool diag = CAUSAL && (col0 + BS - 1 > diag_t);
             if (tail || diag) {
-                const int lim = CAUSAL ? min(p.Skv - 1, row_g) : (p.Skv - 1);  // last visible column
+                const int lim = CAUSAL ? min(p.Skv - 1, diag_t + row) : (p.Skv - 1);  // last visible column
 #pragma unroll
                 for (int i = 0; i < BS; ++i)
                     if (col0 + i > lim) s[i] = -INFINITY;
             }
         };
         // first step whose scores need the mask (every later one does too)
-        const int j_mask = CAUSAL ? min(p.Skv / BS, (m0 + t * BM) / BS) : p.Skv / BS;
+        const int j_mask = CAUSAL ? min(p.Skv / BS, diag_t / BS) : p.Skv / BS;
         // row maximum of sixteen columns folded into two running maxima (two chains per call site -> four in flight)
         auto max16 = [&](const float (&s)[BS], int q, float& ma, float& mb) {
 #pragma unroll
@@ -914,6 +919,7 @@ static int launch_cfg(const AttnArgs& a, cudaStream_t stream, int* launches) {
     p.q_sb = a.qs[0] * C::QB, p.q_sh = a.qs[1] * C::QB, p.q_sr = a.qs[2] * C::QB;
     p.B = a.B, p.Hq = a.Hq, p.Hkv = a.Hkv, p.Sq = a.Sq, p.Skv = a.Skv;
     p.causal = a.causal;
+    p.off = a.causal == QA_CAUSAL_BOTTOM_RIGHT ? a.Skv - a.Sq : 0;
     p.sm_scale_log2 = a.sm_scale * kLog2e;
     p.out_fp16 = (a.out_dtype == QA_DT_FP16);
     p.qk_fp16 = (a.qk_dtype == QA_DT_FP16);

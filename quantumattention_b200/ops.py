@@ -70,7 +70,7 @@ def attention_native(query, key, value, is_causal=False, scale=None, return_lse=
     if query.dtype not in (torch.float16, torch.bfloat16) or key.dtype != query.dtype or value.dtype != query.dtype:
         raise ValueError("attention_forward expects query, key and value of one dtype, torch.float16 or torch.bfloat16")
     sm_scale = (1.0 / math.sqrt(query.size(-1))) if scale is None else float(scale)
-    return _native.attn_fwd(query, key, value, is_causal=is_causal, sm_scale=sm_scale, return_lse=return_lse)
+    return _native.attn_fwd(query, key, value, is_causal=bool(is_causal), sm_scale=sm_scale, return_lse=return_lse)
 
 
 def _scale_mode_of(scale_q: torch.Tensor, query: torch.Tensor, scale_k: Optional[torch.Tensor] = None,
@@ -120,7 +120,7 @@ def fp8_attention_native(query, key, value, scale_q, scale_k, is_causal=False, s
     if out_dtype is None:
         out_dtype = value.dtype if value.dtype in (torch.float16, torch.bfloat16) else torch.bfloat16
     return _native.fp8_attn_fwd(query, key, v_in, scale_q, scale_k, scale_v, scale_mode=scale_mode,
-                                is_causal=is_causal, sm_scale=sm_scale, p_mode=mode, out_dtype=out_dtype,
+                                is_causal=bool(is_causal), sm_scale=sm_scale, p_mode=mode, out_dtype=out_dtype,
                                 return_lse=return_lse)
 
 

@@ -17,7 +17,11 @@ src/quantum_attn/tk/attention.py:417,465); callers such as ParaAttention shard t
   the other ranks' peer-mapped buffers by the copy engines (``qa_copy_2d``), which crosses NVSwitch without taking
   an SM from the attention kernel.  Strategy ``ring``: neighbour ``batch_isend_irecv`` while the fused kernel attends
   the block already here, partial results combined through their log-sum-exp by ``qa_merge_partials``.
-  Non-causal only (as the BASELINE config).
+  The gather strategy also serves GQA (only the Hkv heads of K / V travel) and causal attention over ZIG-ZAG shards:
+  the sequence is cut into 2N chunks and rank r holds chunk r followed by chunk 2N-1-r (``zigzag_shard``), which gives
+  every rank the same causal work.  K / V are gathered in global token order, and each head group is attended in two
+  launches - one per local chunk - whose causal diagonal sits at the END of the keys that chunk sees (the
+  bottom-right alignment of the C ABI, QA_CAUSAL_BOTTOM_RIGHT).  The ring strategy is non-causal and MHA only.
 
 The kernels are reached through a small backend object so that the host logic (ring order, buffer rotation, scale
 exchange, merge order) can be exercised on CPU with the ``gloo`` backend in tests; the default backend is the
@@ -85,8 +89,9 @@ class NativeBackend:
         outs, _ = _native.quantize_fp8(list(tensors), _native.QA_SCALE_HEAD_GIVEN, scales=list(scales), outs=outs)
         return outs
 
-    def attend(self, q8, k8, v, sq, sk, sv, sm_scale, p_mode, out_dtype, out=None, return_lse=True, gate=None):
-        return _native.fp8_attn_fwd(q8, k8, v, sq, sk, sv, scale_mode=_native.QA_SCALE_HEAD, is_causal=False,
+    def attend(self, q8, k8, v, sq, sk, sv, sm_scale, p_mode, out_dtype, out=None, return_lse=True, gate=None, causal=0):
+        """``causal``: 0, QA_CAUSAL_TOP_LEFT or QA_CAUSAL_BOTTOM_RIGHT (include/qattn.h)."""
+        return _native.fp8_attn_fwd(q8, k8, v, sq, sk, sv, scale_mode=_native.QA_SCALE_HEAD, is_causal=causal,
                                     sm_scale=sm_scale, p_mode=p_mode, out_dtype=out_dtype, return_lse=return_lse, out=out,
                                     gate=gate)
 
@@ -116,6 +121,32 @@ def _mark(label: str, device) -> None:
 
 SEQ_STRATEGIES = ("gather", "ring")
 SEQ_TRANSPORTS = ("auto", "nccl", "peer")
+
+
+def zigzag_shard(x: torch.Tensor, world: int, rank: int) -> torch.Tensor:
+    """Rank ``rank``'s shard of a global [B, H, S, D] sequence for causal sequence sharding: dim 2 cut into 2 * world
+    chunks of c = S / (2 * world) tokens, rank r holding chunk r followed by chunk 2 * world - 1 - r ([B, H, 2c, D]).
+    Row i of a causal problem attends i + 1 keys, so chunk j costs ~ (j + 1/2) c^2 and every rank's pair of chunks
+    costs the same 2 * world * c^2."""
+    if world < 1 or not (0 <= rank < world):
+        raise ValueError(f"bad rank {rank} for world size {world}")
+    S = x.shape[2]
+    if S % (2 * world):
+        raise ValueError(f"zigzag_shard: the sequence length {S} must be a multiple of 2 * world = {2 * world}")
+    c = S // (2 * world)
+    return torch.cat([x[:, :, rank * c:(rank + 1) * c], x[:, :, (2 * world - 1 - rank) * c:(2 * world - rank) * c]], 2)
+
+
+def zigzag_unshard(shards: Sequence[torch.Tensor]) -> torch.Tensor:
+    """Inverse of ``zigzag_shard``: the [B, H, 2c, D] shards of ranks 0 .. N-1 -> the global [B, H, 2Nc, D] sequence."""
+    world = len(shards)
+    c = shards[0].shape[2] // 2
+    chunks = [None] * (2 * world)
+    for r, t in enumerate(shards):
+        if t.shape[2] != 2 * c:
+            raise ValueError("zigzag_unshard: every shard must have the same even length")
+        chunks[r], chunks[2 * world - 1 - r] = t[:, :, :c], t[:, :, c:]
+    return torch.cat(chunks, 2)
 
 
 def seq_pv_mode() -> str:
@@ -186,7 +217,13 @@ def head_chunks(B: int, H: int, S_local: int, n_sms: int = 148, max_chunks: int 
     B * hc * ceil(S_local / 256) CTAs (two 128-row query tiles per CTA, one CTA per SM).  ``hc`` is the SMALLEST head
     count (most groups, so the transfer of group i + 1 hides under the attention of group i and the exposed first
     transfer is short) among those whose launch wastes the least of its last wave - no launch then pays more wave
-    quantisation than a single launch over all heads would.  At most ``max_chunks`` groups."""
+    quantisation than a single launch over all heads would.  At most ``max_chunks`` groups.
+
+    ``ring_fp8_attention`` passes the kv heads as ``H`` and B * (Hq / Hkv) as ``B`` (a group of kv heads attends all
+    their query heads in one launch).  Causal calls pass S_local / 2: a group is attended in two launches of one zig-zag
+    chunk each, which have the same CTA count; their CTAs do different work (rank r's first chunk sees (r + 1) chunks of
+    keys, its second 2N - r), so the sizing fills the waves by CTA count only, as it does for the causal diagonal
+    inside any one launch."""
     ctas_per_head = max(1, B * ((S_local + 255) // 256))
     best = None
     for hc in range(1, H + 1):
@@ -291,13 +328,15 @@ class PeerGather:
             st.wait_event(ready)
         self.cur, self.phase = self.phase, self.phase ^ 1
 
-    def pull_group(self, lo: int, hi: int, gate_index: Optional[int] = None) -> List[torch.cuda.Event]:
+    def pull_group(self, lo: int, hi: int, gate_index: Optional[int] = None, zigzag: bool = False) -> List[torch.cuda.Event]:
         """Start the pulls of heads [lo, hi) from every rank (own block: a local copy); returns the events to wait for -
         or, with ``gate_index``, sets the group's words of ``self.flags`` behind the copies instead (gated launch).
         The copies are dealt round-robin to a few streams so that transfers from different peers overlap; the argument
         arrays of a (slot, head range) are marshalled once and re-issued with one call of the C ABI - the host cost of
-        issuing the copies is what the first head group's transfer hides behind, so it has to be small."""
-        key = (self.cur, lo, hi, gate_index is not None)
+        issuing the copies is what the first head group's transfer hides behind, so it has to be small.
+        ``zigzag``: the blocks are zig-zag shards (``zigzag_shard``), and their two halves go to their places in global
+        token order - two copy rows per rank-block."""
+        key = (self.cur, lo, hi, gate_index is not None, zigzag)
         batch = self.batches.get(key)
         if batch is None:
             B, H, S_all, D = self.k_all.shape
@@ -313,13 +352,19 @@ class PeerGather:
             for i in range(1 if gate_index is not None else 0, self.world):
                 r = (self.rank + i) % self.world  # own block first, then the peers - every rank in another order
                 src = self.peer_ptrs[r] + base
-                for b in range(B):
-                    # rows = heads of the group; a row is this rank-block of one head: S x D bytes of K, S x Dv of V
-                    copies.append((k_dst + ((b * H + lo) * S_all + r * S) * D, S_all * D, src + (b * H + lo) * S * D,
-                                   S * D, S * D, hi - lo, raws[n % len(raws)]))
-                    copies.append((v_dst + ((b * H + lo) * S_all + r * S) * Dv, S_all * Dv,
-                                   src + self.nk + (b * H + lo) * S * Dv, S * Dv, S * Dv, hi - lo, raws[(n + 1) % len(raws)]))
-                    n += 2
+                # (first row of the block, first row in the per-head layout, rows): the whole block at r * S, or its
+                # zig-zag halves at chunks r and 2N - 1 - r
+                c = S // 2
+                segs = [(0, r * c, c), (c, (2 * self.world - 1 - r) * c, c)] if zigzag else [(0, r * S, S)]
+                for s0, d0, rows in segs:
+                    for b in range(B):
+                        # rows = heads of the group; a row is this rank-block of one head: rows x D bytes of K, x Dv of V
+                        copies.append((k_dst + ((b * H + lo) * S_all + d0) * D, S_all * D,
+                                       src + ((b * H + lo) * S + s0) * D, S * D, rows * D, hi - lo, raws[n % len(raws)]))
+                        copies.append((v_dst + ((b * H + lo) * S_all + d0) * Dv, S_all * Dv,
+                                       src + self.nk + ((b * H + lo) * S + s0) * Dv, S * Dv, rows * Dv, hi - lo,
+                                       raws[(n + 1) % len(raws)]))
+                        n += 2
             batch = self.batches[key] = _native.CopyBatch(copies)
         batch.issue()
         if gate_index is not None:
@@ -348,16 +393,21 @@ class PeerGather:
         return [self.pull_group(lo, hi) for lo, hi in chunks]
 
 
-def ring_fp8_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, *, scale: Optional[float] = None,
-                       pv_mode: Optional[str] = None, group=None, backend=None,
+def ring_fp8_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, *, is_causal: bool = False,
+                       scale: Optional[float] = None, pv_mode: Optional[str] = None, group=None, backend=None,
                        strategy: Optional[str] = None, transport: Optional[str] = None,
                        head_groups: Optional[int] = None) -> torch.Tensor:
-    """Non-causal FP8 attention over a sequence sharded across the ranks of ``group``.
+    """FP8 attention over a sequence sharded across the ranks of ``group``.
 
-    q, k, v: this rank's [B, H, S_local, D] 16-bit slices (equal S_local on every rank); returns the [B, H, S_local, D]
-    output rows of the local queries against the keys/values of ALL ranks.  With world size 1 this is exactly
-    ``fp8_attn_func(q, k, v)`` in the chosen P mode (the configured one when none is given; every mode is supported:
-    in "16bit" the value blocks travel in 16 bits).
+    q, k, v: this rank's [B, Hq, S_local, D] / [B, Hkv, S_local, D] 16-bit slices (equal S_local on every rank;
+    Hq = Hkv with the ring strategy, a multiple of it with the gather strategy); returns the [B, Hq, S_local, D] output
+    rows of the local queries against the keys/values of ALL ranks.  Non-causal: the slices are contiguous shards of
+    the sequence (rank r holds tokens [r * S_local, (r + 1) * S_local)).  ``is_causal``: the slices are ZIG-ZAG shards
+    (``zigzag_shard``; S_local even), each local query attends the keys up to its own global position (top-left
+    causal attention over the whole sequence), and the output rows come back in the same zig-zag order
+    (``zigzag_unshard`` reassembles the sequence).  With world size 1 this is exactly ``fp8_attn_func(q, k, v,
+    is_causal=is_causal)`` in the chosen P mode (the configured one when none is given; every mode is supported: in
+    "16bit" the value blocks travel in 16 bits).
 
     ``strategy`` "gather" (default): per group of heads, all ranks' K / V blocks are laid end to end in local memory
     and attended in ONE launch over all keys - no partial results; group i + 1 travels while group i is attended.
@@ -365,48 +415,75 @@ def ring_fp8_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, *, sca
     symmetric memory; no SM is spent on communication).  ``head_groups`` overrides the number of head groups
     (default: ``head_chunks``).  ``strategy`` "ring": world - 1 neighbour exchanges, one launch and one (O, LSE) merge
     per block.  Same quantised bytes every way.
+
+    Causal calls (gather strategy only): K / V are laid out in global token order, and each head group is attended in
+    two launches, one per local chunk, against the keys up to that chunk's end - (r + 1) c and (2N - r) c keys for
+    chunk size c = S_local / 2 - with the causal diagonal aligned to the last key (QA_CAUSAL_BOTTOM_RIGHT).  They use
+    per-group launches synchronised by events, never the gated launch.
     """
     be = backend if backend is not None else NativeBackend()
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     rank = dist.get_rank(group) if dist.is_initialized() else 0
-    if q.dim() != 4 or k.shape != v.shape or q.shape[:2] != k.shape[:2] or q.shape[3] != k.shape[3]:
-        raise ValueError("ring_fp8_attention: q, k, v must be [B,H,S_local,D] with equal B, H, D (no GQA)")
+    strategy = default_seq_strategy() if strategy is None else strategy
+    if strategy not in SEQ_STRATEGIES:
+        raise ValueError(f"strategy must be one of {SEQ_STRATEGIES} but got {strategy!r}")
+    if strategy == "ring":
+        if q.dim() != 4 or k.shape != v.shape or q.shape[:2] != k.shape[:2] or q.shape[3] != k.shape[3]:
+            raise ValueError("ring_fp8_attention: q, k, v must be [B,H,S_local,D] with equal B, H, D (no GQA)")
+        if is_causal:
+            raise ValueError("ring_fp8_attention: the ring strategy is non-causal only; use strategy='gather'")
+    elif (q.dim() != 4 or k.dim() != 4 or k.shape != v.shape or q.shape[0] != k.shape[0] or q.shape[2:] != k.shape[2:]
+          or q.shape[1] % k.shape[1]):
+        raise ValueError("ring_fp8_attention: q, k, v must be [B,Hq,S_local,D], [B,Hkv,S_local,D] with Hq a multiple "
+                         "of Hkv")
+    if is_causal and world > 1 and q.shape[2] % 2:
+        raise ValueError(f"ring_fp8_attention: a causal zig-zag shard holds two equal chunks, so S_local must be even "
+                         f"(got {q.shape[2]})")
     if pv_mode is None:
         pv_mode = seq_pv_mode()
     p_mode = ops.pv_mode_code(pv_mode)
     v16 = p_mode == _native.QA_P_16BIT
-    strategy = default_seq_strategy() if strategy is None else strategy
-    if strategy not in SEQ_STRATEGIES:
-        raise ValueError(f"strategy must be one of {SEQ_STRATEGIES} but got {strategy!r}")
     transport = default_seq_transport() if transport is None else transport
     if transport not in SEQ_TRANSPORTS:
         raise ValueError(f"transport must be one of {SEQ_TRANSPORTS} but got {transport!r}")
-    B, H, S, D = q.shape
+    B, Hq, S, D = q.shape
+    H = k.shape[1]  # kv heads: what travels, and what head groups are made of
+    g = Hq // H     # query heads per kv head (GQA): group [lo, hi) attends query heads [lo * g, hi * g)
     sm_scale = (1.0 / math.sqrt(D)) if scale is None else float(scale)
 
-    # 1. head scales of the WHOLE sequence: local scales, one MAX all-reduce (scale is monotone in amax)
+    # 1. head scales of the WHOLE sequence: local scales, one MAX all-reduce (scale is monotone in amax) over the
+    #    [B,Hq] and [B,Hkv] scales laid end to end
     if q.is_cuda:
         _mark("start", q.device)
-    scales = torch.stack(be.local_scales([q, k] if v16 else [q, k, v]))  # [2 or 3, B, H] fp32
+    kv_in = [k] if v16 else [k, v]
+    local = be.local_scales([q] + kv_in) if g == 1 else be.local_scales([q]) + be.local_scales(kv_in)
+    scales = torch.cat([t.reshape(-1) for t in local])  # fp32 [B*Hq + (1 or 2) * B*Hkv]
     if q.is_cuda:
         _mark("amax", q.device)
     if world > 1:
         dist.all_reduce(scales, op=dist.ReduceOp.MAX, group=group)
-    sq, sk, sv = scales[0], scales[1], (None if v16 else scales[2])
+    n_sq, n_sk = B * Hq, B * H
+    sq, sk = scales[:n_sq].view(B, Hq), scales[n_sq:n_sq + n_sk].view(B, H)
+    sv = None if v16 else scales[n_sq + n_sk:].view(B, H)
     out = torch.empty_like(q)
     if q.is_cuda:
         _mark("scales", q.device)
+    causal_kw = {"causal": _native.QA_CAUSAL_TOP_LEFT} if is_causal else {}
 
     if world == 1:
-        q8, k8 = be.quantize([q, k], [sq, sk])
+        if g == 1:
+            q8, k8 = be.quantize([q, k], [sq, sk])
+        else:
+            (q8,), (k8,) = be.quantize([q], [sq]), be.quantize([k], [sk])
         v_in = v if v16 else be.quantize([v], [sv])[0]
-        be.attend(q8, k8, v_in, sq, sk, sv, sm_scale, p_mode, q.dtype, out=out, return_lse=False)
+        be.attend(q8, k8, v_in, sq, sk, sv, sm_scale, p_mode, q.dtype, out=out, return_lse=False, **causal_kw)
         return out
 
     if strategy == "gather":
         # 2. K / V first - they travel - then Q while the first blocks are on the wire
+        c = S // 2 if is_causal else S  # query rows per launch
         if head_groups is None:
-            chunks = head_chunks(B, H, S)
+            chunks = head_chunks(B * g, H, c)
         else:  # caller's choice (tests; tuning)
             hc = -(-H // max(1, min(H, int(head_groups))))
             chunks = [(lo, min(H, lo + hc)) for lo in range(0, H, hc)]
@@ -420,7 +497,8 @@ def ring_fp8_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, *, sca
                 vb.view(v.dtype).copy_(v)
             else:
                 be.quantize([k, v], [sk, sv], outs=[kb, vb])
-            gated = seq_gated_launch(B, H, S) and len(chunks) <= 64
+            # (causal: per-group launches - the two chunks of a group need launches of their own)
+            gated = not is_causal and seq_gated_launch(B * g, H, S) and len(chunks) <= 64
             if gated:
                 comm.flags.zero_()  # (on the calling stream, ahead of the event the copy streams wait for)
             comm.start()
@@ -445,7 +523,7 @@ def ring_fp8_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, *, sca
                     out.copy_(o)
                 _mark("attend", q.device)
                 return out
-            fetch = lambda lo, hi: comm.pull_group(lo, hi)
+            fetch = lambda lo, hi: comm.pull_group(lo, hi, zigzag=is_causal)
 
             def wait(evs):
                 for ev in evs:
@@ -458,8 +536,27 @@ def ring_fp8_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, *, sca
                 k8, v_send = be.quantize([k, v], [sk, sv])
             k_all = torch.empty((B, H, world * S, D), dtype=f8, device=q.device)
             v_all = torch.empty((B, H, world * S, D), dtype=v_send.dtype, device=q.device)
-            fetch = lambda lo, hi: _nccl_gather_heads([k8, v_send], [k_all, v_all], lo, hi, group)
-            wait = lambda w: w.wait()
+            if not is_causal:
+                fetch = lambda lo, hi: _nccl_gather_heads([k8, v_send], [k_all, v_all], lo, hi, group)
+                wait = lambda w: w.wait()
+            else:
+                # zig-zag halves: the first halves (chunks 0 .. N-1) land in rank order straight in place; the second
+                # halves (chunk 2N-1-r of rank r) arrive in rank order, i.e. reversed, in a side buffer and are put in
+                # place by one strided copy per tensor (index_copy_ with the reversed rank order) once they are there
+                tails = [torch.empty((B, H, world * c, D), dtype=t.dtype, device=q.device) for t in (k8, v_send)]
+                rev = torch.arange(world - 1, -1, -1, device=q.device)
+
+                def fetch(lo, hi):
+                    return lo, hi, _nccl_gather_heads(
+                        [k8[:, :, :c], v_send[:, :, :c], k8[:, :, c:], v_send[:, :, c:]],
+                        [k_all[:, :, :world * c], v_all[:, :, :world * c]] + tails, lo, hi, group)
+
+                def wait(pending):
+                    lo, hi, w = pending
+                    w.wait()
+                    for dst, tail in zip((k_all, v_all), tails):  # (as bytes: index_copy_ has no float8 kernels)
+                        dst[:, lo:hi, world * c:].view(torch.uint8).view(B, hi - lo, world, c, -1).index_copy_(
+                            2, rev, tail[:, lo:hi].view(torch.uint8).view(B, hi - lo, world, c, -1))
         # the first group's transfer is started at once; every later one right before the attention of the group in
         # front of it is launched, so the host never spends more than one group's worth of issue time ahead of a launch
         pending = fetch(*chunks[0])
@@ -468,18 +565,30 @@ def ring_fp8_attention(q: torch.Tensor, k: torch.Tensor, v: torch.Tensor, *, sca
         (q8,) = be.quantize([q], [sq])
         if q.is_cuda:
             _mark("quant_q", q.device)
-        # 3. one launch per head group over ALL keys, as its blocks land
+        # 3. one launch per head group over ALL keys (causal: two, one per zig-zag chunk), as its blocks land
         for i, (lo, hi) in enumerate(chunks):
             nxt = fetch(*chunks[i + 1]) if i + 1 < len(chunks) else None
             wait(pending)
             pending = nxt
             if q.is_cuda:
                 _mark("wait", q.device)
-            dst = out[:, lo:hi] if B == 1 else None  # (a head range of a [1,H,S,D] tensor is dense)
-            o = be.attend(q8[:, lo:hi], k_all[:, lo:hi], v_all[:, lo:hi], sq[:, lo:hi], sk[:, lo:hi],
-                          None if v16 else sv[:, lo:hi], sm_scale, p_mode, q.dtype, out=dst, return_lse=False)
-            if dst is None:
-                out[:, lo:hi].copy_(o)
+            qh = slice(lo * g, hi * g)
+            sv_g = None if v16 else sv[:, lo:hi]
+            if not is_causal:
+                dst = out[:, qh] if B == 1 else None  # (a head range of a [1,H,S,D] tensor is dense)
+                o = be.attend(q8[:, qh], k_all[:, lo:hi], v_all[:, lo:hi], sq[:, qh], sk[:, lo:hi], sv_g, sm_scale,
+                              p_mode, q.dtype, out=dst, return_lse=False)
+                if dst is None:
+                    out[:, qh].copy_(o)
+            else:
+                # chunk r sees the keys of chunks 0 .. r, chunk 2N-1-r those of chunks 0 .. 2N-1-r: each the keys up to
+                # its own end, diagonal at the last key.  The kernel writes dense rows; a chunk of a head is not, so
+                # its c x D output is copied into place.
+                for rows, n_keys in ((slice(0, c), (rank + 1) * c), (slice(c, S), (2 * world - rank) * c)):
+                    o = be.attend(q8[:, qh, rows], k_all[:, lo:hi, :n_keys], v_all[:, lo:hi, :n_keys], sq[:, qh],
+                                  sk[:, lo:hi], sv_g, sm_scale, p_mode, q.dtype, return_lse=False,
+                                  causal=_native.QA_CAUSAL_BOTTOM_RIGHT)
+                    out[:, qh, rows].copy_(o)
             if q.is_cuda:
                 _mark("attend", q.device)
         return out
